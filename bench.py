@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- SELA hot path on B200: encode + decode MSamples/s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A step = one pass of the hot path over one batch: fused encode of the batch (PCM ->
@@ -395,6 +395,32 @@ def make_pcm(seed):
     return synth.sine_noise(SAMPLE_RATE, CHANNELS, seconds=SECONDS, seed=seed)
 
 
+DUMP_FRAMES = 1024
+
+
+def dump_outputs(path, descs, words, pcm_out):
+    """--dump-outputs: what a caller of the timed path received from its last step, so that two builds can be
+    compared output for output.  The workload's words and PCM run to hundreds of MB, so those two files hold a
+    fixed sample of frames (seed 0; it depends only on the frame count), in frame order:
+      descs.npy        float64 [subframes, 12]     every descriptor, fields in DESC_DTYPE order
+      words.npy        float64 [n]                 each sampled frame's Rice words, subframe by subframe
+      pcm_decoded.npy  float32 [frames*2048, ch]   the decoded PCM of the sampled frames"""
+    n_frames = pcm_out.size // (FRAME * CHANNELS)
+    frames = np.sort(np.random.default_rng(0).choice(n_frames, min(n_frames, DUMP_FRAMES), replace=False))
+    sub = (frames[:, None] * CHANNELS + np.arange(CHANNELS)).reshape(-1)
+    spans = [(int(descs[i][o]), int(descs[i][n])) for i in sub
+             for o, n in (("refl_offset", "refl_words"), ("res_offset", "res_words"))]
+    out = {
+        "descs": np.stack([descs[f].astype(np.float64) for f in descs.dtype.names], axis=1),
+        "words": np.concatenate([words[a:a + n] for a, n in spans]).astype(np.float64),
+        "pcm_decoded": pcm_out.reshape(n_frames, FRAME, CHANNELS)[frames].reshape(-1, CHANNELS).astype(np.float32),
+    }
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_reference_leg(pcm, target_seconds=8.0):
     """Time the reference's multithreaded CPU coder on a bounded sample of the workload."""
     import oracle_lib as ol
@@ -544,6 +570,9 @@ def run_ours(args, rank, world, local_rank):
     enc_ms = statistics.fmean(ev[2 * i].elapsed_time(ev[2 * i + 1]) for i in range(args.steps))
     dec_ms = statistics.fmean(ev[2 * i + 1].elapsed_time(ev[2 * i + 2]) for i in range(args.steps))
     codec.check_status()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, codec.descs.cpu().numpy().view(_lib.DESC_DTYPE),
+                     codec.words[:int(codec.words_used.item())].cpu().numpy().view(np.uint32), out.cpu().numpy())
 
     # ---------------- end-to-end leg (host buffers through the public C ABI) ----------------
     def pinned(nbytes, dtype):
@@ -570,7 +599,7 @@ def run_ours(args, rank, world, local_rank):
         split[0] += t_b - t_a
         split[1] += time.perf_counter() - t_b
 
-    e2e_steps = max(3, min(args.steps, 20))
+    e2e_steps = args.steps
     for _ in range(3):
         e2e_step()
     if dist:
@@ -705,7 +734,13 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="skip the configs[3]/[4] block (profiling runs)")
     ap.add_argument("--sharded-minutes", type=int, default=0, help="length of the config-4 file (default 60)")
     ap.add_argument("--sharded-timeout", type=int, default=240, help="seconds before the sharded block is given up (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm codes a sample sized by a timing probe, not a fixed input")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

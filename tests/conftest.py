@@ -1,8 +1,6 @@
 import pathlib
 import sys
 
-import pytest
-
 ROOT = pathlib.Path(__file__).resolve().parent.parent
 for p in (str(ROOT), str(ROOT / "tests")):
     if p not in sys.path:
@@ -11,14 +9,8 @@ for p in (str(ROOT), str(ROOT / "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "ref: needs oracle/_ref (the compiled reference; built where /root/reference exists)")
 
 
 def pytest_collection_modifyitems(config, items):
     import oracle_lib
     oracle_lib.build()
-    if not oracle_lib.have_ref():
-        skip = pytest.mark.skip(reason="oracle/_ref/libsela_ref.so not built (no /root/reference here)")
-        for it in items:
-            if "ref" in it.keywords:
-                it.add_marker(skip)

@@ -1,32 +1,52 @@
 #!/usr/bin/env python3
 """Generate the golden vectors under tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container (needs /root/reference; builds oracle/_ref via oracle/Makefile):
+    python tests/golden/make_golden.py <reference checkout> [frames] [stages] [cli]
 
-    python tests/golden/make_golden.py
-
+builds oracle/_ref from that checkout (oracle/Makefile) and writes the files named (default: all).
 The reference ships no golden files (SURVEY.md 4), so these are outputs of the reference's own
-classes (frame::FrameEncoder / FrameDecoder through oracle/ref_shim.cpp) on seeded inputs.
-They travel to the GPU box, where /root/reference does not exist.
+classes (through oracle/ref_shim.cpp) and CLI (oracle/ref_cli_main.cpp) on seeded inputs.
+They let the tests compare with the reference on machines that do not have it.
 
   golden_frames.npz
     pcm_<case>      int16 [n_frames*2048, channels]   input
     descs_<case>    structured (32-byte descriptor)   reference encoder output
     words_<case>    uint32                            reference encoder output (arena)
     decoded_<case>  int16                             reference DECODER output for (descs, words)
+
+  reference_stages.npz   (tests/test_oracle_vs_ref.py, tests/test_host_logic.py)
+    fam_<name>_*           LPC analysis, Rice streams and decodes of signals.families()
+    rand_*, dc_*           order / coefficients / residue digest of signals.random_frames(300, 11), DC frames
+    rice_<i>_*             Rice parameter, words and decode of test_oracle_vs_ref.rice_inputs()
+    batch<ch>_*            descriptors, word digest and decode digest of test_oracle_vs_ref.batch_pcm(ch)
+    lpc_first_order_bits   uint64[128]: the reference's firstOrderCoefficients as IEEE-754 bit patterns
+
+  reference_cli.npz      (tests/test_host_cli.py, tests/test_container.py, tests/test_multi_device.py)
+    <case>_sela, _wav      digests of what the reference CLI's -e wrote for test_host_cli._cases(), and of
+                           what its -d wrote for that .sela
+    pack_<ch>_sela         digest of its -e output for test_container.pack_cases()
+    oct700_sela, _wav      digests of its -e / -d output for the 700-frame 8-channel WAV
+
+Digests are oracle_lib.digest (SHA-256 over dtype and bytes, 128 bits): they stand for outputs too
+large to keep, so a mismatch says only that the bytes differ.
 """
 import pathlib
+import re
+import struct
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
-ROOT = pathlib.Path(__file__).resolve().parent.parent.parent
+HERE = pathlib.Path(__file__).resolve().parent
+ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "tests"))
 
 import oracle_lib as ol  # noqa: E402
 import signals  # noqa: E402
-from sela_b200 import synth  # noqa: E402
+from sela_b200 import synth, wavio  # noqa: E402
 
 
 def cases():
@@ -52,10 +72,7 @@ def cases():
     return out
 
 
-def main():
-    assert ol.have_ref() or pathlib.Path("/root/reference").exists(), "needs the reference tree"
-    R = ol.load("ref")
-    assert R.kind == "reference"
+def frames(R):
     blob = {}
     for name, pcm in cases().items():
         ch = pcm.shape[1]
@@ -66,7 +83,91 @@ def main():
         blob["decoded_" + name] = R.decode_frames(descs, words, ch)
         print("%-14s ch=%d frames=%d words=%d lossless=%s" % (
             name, ch, pcm.shape[0] // 2048, words.size, np.array_equal(blob["decoded_" + name], pcm.reshape(-1))))
-    np.savez_compressed(pathlib.Path(__file__).parent / "golden_frames.npz", **blob)
+    return blob
+
+
+def _padded_q(q):
+    out = np.zeros(100, np.int32)
+    out[:q.size] = q
+    return out
+
+
+def stages(R, ref_tree):
+    import test_oracle_vs_ref as t
+    blob = {}
+    for name, s in signals.families().items():
+        a = R.lpc_analyse(s)
+        kq, wq = R.rice_encode(a["q"])
+        kr, wr = R.rice_encode(a["res"])
+        p = "fam_%s_" % name
+        blob.update({p + "order": a["order"], p + "q": a["q"], p + "c": a["c"], p + "res": a["res"],
+                     p + "kq": kq, p + "wq": wq, p + "kr": kr, p + "wr": wr,
+                     p + "decoded_q": ol.digest(R.rice_decode(wq, kq, a["q"].size)),
+                     p + "decoded_r": ol.digest(R.rice_decode(wr, kr, a["res"].size)),
+                     p + "synthesised": ol.digest(R.lpc_synthesise(a["res"], a["order"], a["q"]))})
+    for key, frames_ in (("rand", signals.random_frames(300, seed=11)),
+                         ("dc", [np.full(2048, v, np.int32) for v in t.dc_levels()])):
+        an = [R.lpc_analyse(s) for s in frames_]
+        blob[key + "_order"] = np.array([a["order"] for a in an], np.int32)
+        blob[key + "_q"] = np.stack([_padded_q(a["q"]) for a in an])
+        blob[key + "_res"] = np.array([ol.digest(a["res"]) for a in an])
+    blob["dc_level"] = np.array(t.dc_levels(), np.int32)
+    for i, x in enumerate(t.rice_inputs()):
+        k, w = R.rice_encode(x)
+        blob["rice_%d_k" % i], blob["rice_%d_words" % i] = k, w
+        blob["rice_%d_decoded" % i] = ol.digest(R.rice_decode(w, k, x.size))
+    for ch in (1, 2, 3, 8):
+        d, w = R.encode_frames(t.batch_pcm(ch), ch)
+        blob["batch%d_descs" % ch], blob["batch%d_words" % ch] = d, ol.digest(w)
+        blob["batch%d_decoded" % ch] = ol.digest(R.decode_frames(d, w, ch))
+    text = (ref_tree / "src" / "include" / "lpc.hpp").read_text()
+    m = re.search(r"firstOrderCoefficients\[128\]\s*=\s*\{([^}]*)\}", text)
+    vals = [float(v) for v in m.group(1).replace("\n", " ").split(",") if v.strip()]
+    assert len(vals) == 128
+    blob["lpc_first_order_bits"] = np.array([struct.unpack("<Q", struct.pack("<d", v))[0] for v in vals], np.uint64)
+    return blob
+
+
+def cli():
+    import test_container
+    import test_host_cli
+    exe = ROOT / "oracle" / "_ref" / "sela_ref_cli"
+    file_digest = lambda p: ol.digest(np.frombuffer(p.read_bytes(), np.uint8))
+
+    def run(mode, src, dst):
+        subprocess.run([str(exe), mode, str(src), str(dst)], check=True, capture_output=True, timeout=600)
+
+    blob = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        tmp = pathlib.Path(tmp)
+        for name, wav in test_host_cli._cases(tmp).items():
+            run("-e", wav, tmp / "r.sela")
+            run("-d", tmp / "r.sela", tmp / "r.wav")
+            blob[name + "_sela"] = file_digest(tmp / "r.sela")
+            blob[name + "_wav"] = file_digest(tmp / "r.wav")
+        for ch, rate, pcm in test_container.pack_cases():
+            wavio.write_wav(tmp / "in.wav", pcm, rate)
+            run("-e", tmp / "in.wav", tmp / "r.sela")
+            blob["pack_%d_sela" % ch] = file_digest(tmp / "r.sela")
+        wavio.write_wav(tmp / "oct.wav", synth.sine_noise(48000, 8, n_frames=700, seed=2), 48000)
+        run("-e", tmp / "oct.wav", tmp / "r.sela")
+        run("-d", tmp / "r.sela", tmp / "r.wav")
+        blob["oct700_sela"], blob["oct700_wav"] = file_digest(tmp / "r.sela"), file_digest(tmp / "r.wav")
+    return blob
+
+
+def main():
+    ref_tree = pathlib.Path(sys.argv[1]).resolve()
+    which = sys.argv[2:] or ["frames", "stages", "cli"]
+    subprocess.run(["make", "-C", str(ROOT / "oracle"), "SELA_REF=%s" % ref_tree], check=True, capture_output=True)
+    R = ol.load("ref")
+    assert R.kind == "reference"
+    if "frames" in which:
+        np.savez_compressed(HERE / "golden_frames.npz", **frames(R))
+    if "stages" in which:
+        np.savez_compressed(HERE / "reference_stages.npz", **stages(R, ref_tree))
+    if "cli" in which:
+        np.savez_compressed(HERE / "reference_cli.npz", **cli())
 
 
 if __name__ == "__main__":

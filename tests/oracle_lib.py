@@ -6,7 +6,7 @@
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs import this.
 """
 import ctypes as C
-import os
+import hashlib
 import pathlib
 import subprocess
 
@@ -36,9 +36,8 @@ assert DESC_DTYPE.itemsize == C.sizeof(Desc) == 32, (DESC_DTYPE.itemsize, C.size
 
 
 def build(force=False):
-    """make -C oracle (liboracle.so always; _ref only where /root/reference exists)."""
-    if force or not (ORACLE_DIR / "liboracle.so").exists() or (
-            os.path.isdir("/root/reference") and not (ORACLE_DIR / "_ref" / "libsela_ref.so").exists()):
+    """make -C oracle (liboracle.so always; _ref only where the reference sources are present)."""
+    if force or not (ORACLE_DIR / "liboracle.so").exists():
         subprocess.run(["make", "-C", str(ORACLE_DIR)], check=True, capture_output=True)
 
 
@@ -198,6 +197,22 @@ def load(which="port"):
 def best():
     """The strongest checker available: the compiled reference if present, else the port."""
     return load("ref") if have_ref() else load("port")
+
+
+def golden(name):
+    """tests/golden/<name>.npz, loaded once."""
+    if name not in _golden:
+        _golden[name] = np.load(ROOT / "tests" / "golden" / (name + ".npz"))
+    return _golden[name]
+
+
+_golden = {}
+
+
+def digest(a):
+    """Short SHA-256 of an array's dtype and bytes: how tests/golden stores reference outputs too large to keep."""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(a.dtype.str.encode() + a.tobytes()).hexdigest()[:32]
 
 
 def fnv1a32(words):

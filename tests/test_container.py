@@ -12,7 +12,6 @@ import oracle_lib as ol
 from sela_b200 import SelaB200Error, codec, synth, wavio
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
-REF_CLI = ROOT / "oracle" / "_ref" / "sela_ref_cli"
 FRAME = 2048
 
 
@@ -35,19 +34,18 @@ def _blob(O, pcm, channels, rate=44100):
 
 # ------------------------------------------------------------------ CPU --
 
-@pytest.mark.ref
-def test_pack_container_helper_equals_reference_writer(O, tmp_path):
+def pack_cases():
+    """(channels, rate, pcm) of the WAVs the reference CLI encoded for tests/golden/reference_cli.npz."""
+    return [(channels, rate, _stereo(n, 4) if channels == 2 else synth.sine_noise(rate, channels, n_frames=n, seed=6))
+            for channels, rate, n in ((2, 44100, 9), (1, 22050, 4), (8, 48000, 3))]
+
+
+def test_pack_container_helper_equals_reference_writer(O):
     """Pins the test helper itself: oracle frames packed by wavio.pack_container are the bytes the
-    reference CLI writes for the same WAV."""
-    if not REF_CLI.exists():
-        pytest.skip("reference CLI not built")
-    for channels, rate, n in ((2, 44100, 9), (1, 22050, 4), (8, 48000, 3)):
-        pcm = _stereo(n, 4) if channels == 2 else synth.sine_noise(rate, channels, n_frames=n, seed=6)
-        wavio.write_wav(tmp_path / "in.wav", pcm, rate)
-        subprocess.run([str(REF_CLI), "-e", str(tmp_path / "in.wav"), str(tmp_path / "ref.sela")], check=True,
-                       capture_output=True, timeout=300)
+    reference CLI wrote for the same WAV."""
+    for channels, rate, pcm in pack_cases():
         blob, _, _ = _blob(O, pcm, channels, rate)
-        assert blob == (tmp_path / "ref.sela").read_bytes(), channels
+        assert ol.digest(np.frombuffer(blob, np.uint8)) == ol.golden("reference_cli")["pack_%d_sela" % channels], channels
 
 
 def test_container_walk_matches_descriptors(O):

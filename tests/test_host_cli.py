@@ -1,20 +1,22 @@
 """The C++ mirror of the reference interface and the CLI built on it (sela_b200/host).
 
-CPU part: the container code (WAV / .sela readers and writers) against the compiled reference.
-GPU part: `sela -e/-d` byte-for-byte against the reference CLI (oracle/_ref/sela_ref_cli, which
-travels to the GPU box as a prebuilt binary), the reference's own main.cpp linked against this
-library, and the reference's unit tests re-expressed on the mirror classes."""
+CPU part: the container code (WAV / .sela readers and writers) against the reference's file code.
+GPU part: `sela -e/-d` byte-for-byte against the reference CLI, the reference's own main.cpp linked
+against this library, and the reference's unit tests re-expressed on the mirror classes.
+Digests of what the reference CLI wrote for the WAVs of _cases() (the .sela, and the .wav it decodes that
+to) are stored in tests/golden/reference_cli.npz by tests/golden/make_golden.py."""
 import pathlib
+import struct
 import subprocess
 
 import numpy as np
 import pytest
 
+import oracle_lib as ol
 from sela_b200 import synth, wavio
 
 ROOT = pathlib.Path(__file__).resolve().parent.parent
 BIN = ROOT / "sela_b200" / "host" / "bin"
-REF_CLI = ROOT / "oracle" / "_ref" / "sela_ref_cli"
 
 
 def _run(*cmd, ok=True, env=None):
@@ -45,21 +47,36 @@ def _cases(tmp):
     return out
 
 
+def _file_digest(path):
+    return ol.digest(np.frombuffer(path.read_bytes(), np.uint8))
+
+
+def _reference_sela(name, wav):
+    """The .sela bytes the reference CLI writes for `wav`: the CPU oracle's frames in the reference's file layout,
+    checked against the digest of what the reference wrote."""
+    raw = wav.read_bytes()
+    ch, rate = struct.unpack_from("<HI", raw, 22)
+    pcm = np.frombuffer(raw, "<i2", offset=raw.index(b"data") + 8)
+    pcm = pcm[: pcm.size // (2048 * ch) * 2048 * ch]                 # the reference drops the partial last frame
+    blob = wavio.pack_container(*ol.load("port").encode_frames(pcm, ch), rate, ch)
+    assert ol.digest(np.frombuffer(blob, np.uint8)) == ol.golden("reference_cli")[name + "_sela"], name
+    return blob
+
+
 # ------------------------------------------------------------------ CPU --
 
-@pytest.mark.ref
 def test_container_code_matches_reference(tmp_path):
     """file::SelaFile read->write is byte-identical on reference-produced files; file::WavFile
     read->(canonical)write equals what the reference decoder writes back (header + tail drop)."""
     _ensure_built()
+    ref = ol.golden("reference_cli")
     for name, wav in _cases(tmp_path).items():
-        ref_sela, ref_wav = tmp_path / (name + ".ref.sela"), tmp_path / (name + ".ref.wav")
-        _run(REF_CLI, "-e", wav, ref_sela)
-        _run(REF_CLI, "-d", ref_sela, ref_wav)
+        ref_sela = tmp_path / (name + ".ref.sela")
+        ref_sela.write_bytes(_reference_sela(name, wav))
         _run(BIN / "container_check", "sela", ref_sela, tmp_path / "rt.sela")
         assert (tmp_path / "rt.sela").read_bytes() == ref_sela.read_bytes(), name
         _run(BIN / "container_check", "wav", wav, tmp_path / "rt.wav")
-        assert (tmp_path / "rt.wav").read_bytes() == ref_wav.read_bytes(), name
+        assert _file_digest(tmp_path / "rt.wav") == ref[name + "_wav"], name
 
 
 def test_container_errors_match_reference_messages(tmp_path):
@@ -99,18 +116,14 @@ def test_cli_byte_parity_with_reference_cli(tmp_path, binary):
     binary = binary.split("-")[0]
     if not (BIN / binary).exists():
         pytest.skip("%s not built (needs the reference tree at build time)" % binary)
-    have_ref = REF_CLI.exists()
+    ref = ol.golden("reference_cli")
     for name, wav in _cases(tmp_path).items():
         ours_sela, ours_wav = tmp_path / (name + ".sela"), tmp_path / (name + ".out.wav")
         p = _run(BIN / binary, "-e", wav, ours_sela, env=env)
         assert "Encoding: " in p.stdout
         _run(BIN / binary, "-d", ours_sela, ours_wav, env=env)
-        if have_ref:
-            ref_sela, ref_wav = tmp_path / (name + ".ref.sela"), tmp_path / (name + ".ref.wav")
-            _run(REF_CLI, "-e", wav, ref_sela)
-            assert ours_sela.read_bytes() == ref_sela.read_bytes(), name          # bit-identical .sela
-            _run(REF_CLI, "-d", ours_sela, ref_wav)                               # reference decodes ours
-            assert ours_wav.read_bytes() == ref_wav.read_bytes(), name            # bit-identical .wav
+        assert _file_digest(ours_sela) == ref[name + "_sela"], name                # bit-identical .sela
+        assert _file_digest(ours_wav) == ref[name + "_wav"], name                 # bit-identical .wav
         # lossless against the source (whole frames only)
         _, ch, pcm_out = wavio.read_wav_pcm(ours_wav)
         data_at = wav.read_bytes().index(b"data") + 8

@@ -81,13 +81,9 @@ def test_lpc_tables_identical_in_oracle_and_product():
     a = pat.findall((root / "oracle" / "lpc_tables.inc").read_text())
     b = pat.findall((root / "sela_b200" / "csrc" / "lpc_tables.cuh").read_text())
     assert a == b and len(a) == 129
-    ref = pathlib.Path("/root/reference/src/include/lpc.hpp")
-    if ref.exists():     # format constants still match the reference header, bit for bit
-        import struct
-        text = ref.read_text()
-        m = re.search(r"firstOrderCoefficients\[128\]\s*=\s*\{([^}]*)\}", text)
-        vals = [float(t) for t in m.group(1).replace("\n", " ").split(",") if t.strip()]
-        assert ["0x%016xULL" % struct.unpack("<Q", struct.pack("<d", v))[0] for v in vals] == a[:128]
+    # format constants match the reference header's firstOrderCoefficients[128], bit for bit
+    bits = ol.golden("reference_stages")["lpc_first_order_bits"]
+    assert ["0x%016xULL" % int(v) for v in bits] == a[:128]
 
 
 def test_zero_history_bit_exactness_argument():
