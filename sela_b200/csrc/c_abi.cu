@@ -144,68 +144,32 @@ struct PipelineDrain {
     }
 };
 
-// Chunking of the pipelined host-buffer calls: enough chunks to overlap PCIe with compute,
-// each still several waves of warps, workspace bounded for huge batches.
-// `parts`: target number of chunks.  Measured on the BASELINE batch (12 919 stereo frames,
-// tools/e2e_chunk_sweep.py): encode is best at 8 chunks (4.2 ms end to end vs 3.8 ms of kernels);
-// decode at 4 -- its Rice kernel is one lane per stream and latency-bound, so a chunk must still be
-// thousands of streams.
-uint32_t chunk_frames_for(uint32_t n_frames, uint32_t parts)
-{
-    if (const char *env = std::getenv("SELAB200_CHUNK_FRAMES")) { // tuning / tests only
-        long v = std::atol(env);
-        if (v > 0) {
-            uint32_t c = (uint32_t)v;
-            while ((n_frames + c - 1) / c > (uint32_t)kMaxChunks)
-                c *= 2;
-            return c;
-        }
-    }
-    uint32_t c = (n_frames + parts - 1) / parts;
-    if (c < 512) c = 512;
-    if (c > 16384) c = 16384;
-    while ((n_frames + c - 1) / c > (uint32_t)kMaxChunks)
-        c *= 2;
-    return c;
-}
-
-// Chunk boundaries of a pipelined host-buffer call.  Equal chunks; for the encoder the first and
-// the last are cut into shrinking pieces: what its pipeline cannot hide is the upload of the first
-// chunk before any kernel runs and the download of the last chunk after the last kernel, so those
-// two are made small (measured on the BASELINE batch: encode call 4.06 -> 3.93 ms; the decode call,
-// whose small chunks each pay the Rice kernel's fixed latency, gets slower and keeps equal chunks).
-// SELAB200_TAPER=0 switches it off.
+// Chunk boundaries of the pipelined host-buffer calls (encode and both decode paths).  About eight
+// chunks: enough to overlap PCIe with compute, each still several waves of warps, and at most 16 384
+// frames, which bounds the workspace for huge batches (tools/e2e_chunk_sweep.py on a B200, BASELINE
+// batch of 12 919 stereo frames: encode is best at 8 chunks, 4.2 ms end to end vs 3.8 ms of kernels).
+// The first and the last chunk are cut into shrinking pieces: what a pipeline cannot hide is the
+// upload of the first chunk before any kernel runs and the download of the last chunk after the last
+// kernel, so those two are made small (same batch: encode call 4.06 -> 3.93 ms, decode call 3.80 ->
+// 3.67 ms).
 struct ChunkPlan {
     std::vector<uint32_t> start; // n_chunks + 1 boundaries
     uint32_t max_frames = 0;     // largest chunk (sizes the per-lane workspace)
     uint32_t chunks() const { return (uint32_t)start.size() - 1; }
 };
-// decode-side knobs for measurements: SELAB200_DEC_PARTS (target chunk count), SELAB200_DEC_TAPER=1
-uint32_t dec_parts()
-{
-    if (const char *e = std::getenv("SELAB200_DEC_PARTS")) {
-        const long v = std::atol(e);
-        if (v >= 1 && v <= 64)
-            return (uint32_t)v;
-    }
-    return 8;
-}
-bool dec_taper()
-{
-    // round 1 kept equal chunks for decode (small chunks starved the lane-per-stream Rice kernel); with streams cut
-    // into parts for small batches (rice_vs.cuh) the shrinking first and last chunks pay here too: decode call 3.80 -> 3.67 ms
-    const char *e = std::getenv("SELAB200_DEC_TAPER");
-    return !(e && e[0] == '0');
-}
 
-ChunkPlan plan_chunks(uint32_t n_frames, uint32_t parts, bool allow_taper)
+ChunkPlan plan_chunks(uint32_t n_frames)
 {
+    // SELAB200_CHUNK_FRAMES (tests and measurement only): frames per chunk, no shrinking pieces; the tests
+    // use it to push many tiny chunks through the pipelines on small inputs.
+    const char *env = std::getenv("SELAB200_CHUNK_FRAMES");
+    const long forced = env ? std::atol(env) : 0;
+    uint32_t cf = forced > 0 ? (uint32_t)forced : std::min(std::max((n_frames + 7) / 8, 512u), 16384u);
+    while ((n_frames + cf - 1) / cf > (uint32_t)kMaxChunks)
+        cf *= 2;
     ChunkPlan p;
-    const uint32_t cf = chunk_frames_for(n_frames, parts);
     const uint32_t n_base = (n_frames + cf - 1) / cf;
-    const char *env = std::getenv("SELAB200_TAPER");
-    const bool taper = allow_taper && !(env && env[0] == '0') && !std::getenv("SELAB200_CHUNK_FRAMES") && n_base >= 4 &&
-                       n_base + 6 <= (uint32_t)kMaxChunks;
+    const bool taper = !env && n_base >= 4 && n_base + 6 <= (uint32_t)kMaxChunks;
     p.start.push_back(0);
     for (uint32_t c = 0; c < n_base; c++) {
         const uint32_t f0 = c * cf, f1 = (f0 + cf <= n_frames) ? f0 + cf : n_frames, len = f1 - f0;
@@ -388,12 +352,13 @@ int launch_rice_decode(const DecodeParams &p, int which, cudaStream_t stream)
     return launch_check(which ? "k_rice_decode(res)" : "k_rice_decode(refl)");
 }
 
-// Residue streams (K5 proper).  Large batches: one lane per stream through k_rice_decode_vs.  Smaller
+// Residue streams (K5 proper).  Large batches: one lane per stream through k_rice_decode_vc.  Smaller
 // ones: every stream is cut into S parts first (k_rice_split_index), so that a batch of BASELINE's
-// size still fills the machine.  SELAB200_RICE_SPLIT = 0 (first-generation kernel only), 1, 2, 4, 8, 16
-// overrides the choice.  aux: n_sub * 64 bytes (split table + per-stream flags).
+// size still fills the machine.  aux: n_sub * 64 bytes (split table + per-stream flags).
 int rice_split_log2(size_t n_sub)
 {
+    // SELAB200_RICE_SPLIT = 0 (first-generation kernel only), 1, 2, 4, 8, 16 overrides the choice; it exists for
+    // tests and measurement, which reach every S on small inputs.
     if (const char *env = std::getenv("SELAB200_RICE_SPLIT")) {
         const long v = std::atol(env);
         if (v <= 0)
@@ -404,7 +369,7 @@ int rice_split_log2(size_t n_sub)
         return l;
     }
     // Measured on B200 (profiles/r02_rice_decode_roofline.json): from about 12 000 streams up one lane per stream
-    // (S = 1) through k_rice_decode_vs is fastest -- the two split passes cost more than the extra warps bring
+    // (S = 1) through k_rice_decode_vc is fastest -- the two split passes cost more than the extra warps bring
     // once every SM has a few warps of its own; below that the machine is starved and cutting the streams
     // wins (500 streams: S = 16 is 3.5x the first-generation kernel, 8 000 streams: S = 8 is 1.9x).
     if (n_sub >= 12000)
@@ -419,20 +384,10 @@ template <int LOG2S>
 int launch_split_index(const RiceVsParams &q, size_t n_sub, cudaStream_t stream)
 {
     const unsigned blocks = (unsigned)(((n_sub << LOG2S) + 32 * kVsWarps - 1) / (32 * kVsWarps));
-    int geom = 1;
-    if (const char *env = std::getenv("SELAB200_RICE_GEOM_A"))
-        geom = std::atoi(env);
-    if (geom == 1) {
-        constexpr size_t smem = split_smem_bytes<32>();
-        if (int rc = set_smem(k_rice_split_index<LOG2S, 32, 16>, smem))
-            return rc;
-        k_rice_split_index<LOG2S, 32, 16><<<blocks, 32 * kVsWarps, smem, stream>>>(q);
-    } else {
-        constexpr size_t smem = split_smem_bytes<64>();
-        if (int rc = set_smem(k_rice_split_index<LOG2S, 64, 16>, smem))
-            return rc;
-        k_rice_split_index<LOG2S, 64, 16><<<blocks, 32 * kVsWarps, smem, stream>>>(q);
-    }
+    constexpr size_t smem = split_smem_bytes<32>();
+    if (int rc = set_smem(k_rice_split_index<LOG2S, 32, 16>, smem))
+        return rc;
+    k_rice_split_index<LOG2S, 32, 16><<<blocks, 32 * kVsWarps, smem, stream>>>(q);
     return launch_check("k_rice_split_index");
 }
 
@@ -464,74 +419,11 @@ int launch_rice_residues(const DecodeParams &p, void *aux, cudaStream_t stream)
         return rc;
     const size_t n_vs = n_sub << log2s;
     const unsigned vs_blocks = (unsigned)((n_vs + 32 * kVsWarps - 1) / (32 * kVsWarps));
-    // geometry: 3 = rings filled cooperatively, 128-byte segments (default: fastest at every batch size measured);
-    // 0 = per-lane cp.async rings; 1, 2 = the same with half the shared memory; 100+ = ablations (tools/rice_ablation.sh)
-    int geom = 3;
-    if (const char *env = std::getenv("SELAB200_RICE_GEOM"))
-        geom = std::atoi(env);
-    if (geom == 1) {
-        constexpr size_t smem = vs_smem_bytes<32, 16>();
-        if (int rc2 = set_smem(k_rice_decode_vs<32, 16, 16>, smem))
-            return rc2;
-        k_rice_decode_vs<32, 16, 16><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom == 2) {
-        constexpr size_t smem = vs_smem_bytes<32, 32>();
-        if (int rc2 = set_smem(k_rice_decode_vs<32, 16, 32>, smem))
-            return rc2;
-        k_rice_decode_vs<32, 16, 32><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom == 3) { // cooperative rings
-        constexpr size_t smem = vc_smem_bytes<32>();
-        if (int rc2 = set_smem(k_rice_decode_vc<16, 32>, smem))
-            return rc2;
-        k_rice_decode_vc<16, 32><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom == 4) { // cooperative rings, half tile (more warps per SM)
-        constexpr size_t smem = vc_smem_bytes<16>();
-        if (int rc2 = set_smem(k_rice_decode_vc<16, 16>, smem))
-            return rc2;
-        k_rice_decode_vc<16, 16><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom == 5) { // cooperative rings, 256-byte row segments on the way out
-        constexpr size_t smem = vc_smem_bytes<64>();
-        if (int rc2 = set_smem(k_rice_decode_vc<16, 64>, smem))
-            return rc2;
-        k_rice_decode_vc<16, 64><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom == 6) { // 512-byte row segments
-        constexpr size_t smem = vc_smem_bytes<128>();
-        if (int rc2 = set_smem(k_rice_decode_vc<16, 128>, smem))
-            return rc2;
-        k_rice_decode_vc<16, 128><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    } else if (geom >= 200 && geom < 232) { // ablations of the cooperative decoder: 200 + bit mask (8: no copy instruction)
-        constexpr size_t smem = vc_smem_bytes<32>();
-        switch (geom - 200) {
-#define SELAB200_ABL(m)                                                                    \
-    case m:                                                                                \
-        if (int rc2 = set_smem(k_rice_decode_vc<16, 32, m>, smem))                         \
-            return rc2;                                                                    \
-        k_rice_decode_vc<16, 32, m><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s); \
-        break;
-            SELAB200_ABL(1) SELAB200_ABL(2) SELAB200_ABL(3) SELAB200_ABL(4) SELAB200_ABL(5) SELAB200_ABL(6) SELAB200_ABL(7) SELAB200_ABL(8) SELAB200_ABL(12) SELAB200_ABL(16)
-#undef SELAB200_ABL
-        default: break;
-        }
-    } else if (geom >= 100 && geom < 108) { // ablations (measurement only): 100 + bit mask
-        constexpr size_t smem = vs_smem_bytes<64, 32>();
-        switch (geom - 100) {
-#define SELAB200_ABL(m)                                                                        \
-    case m:                                                                                    \
-        if (int rc2 = set_smem(k_rice_decode_vs<64, 16, 32, m>, smem))                         \
-            return rc2;                                                                        \
-        k_rice_decode_vs<64, 16, 32, m><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s); \
-        break;
-            SELAB200_ABL(1) SELAB200_ABL(2) SELAB200_ABL(3) SELAB200_ABL(4) SELAB200_ABL(5) SELAB200_ABL(6) SELAB200_ABL(7)
-#undef SELAB200_ABL
-        default: break;
-        }
-    } else {
-        constexpr size_t smem = vs_smem_bytes<64, 32>();
-        if (int rc2 = set_smem(k_rice_decode_vs<64, 16, 32>, smem))
-            return rc2;
-        k_rice_decode_vs<64, 16, 32><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
-    }
-    if (int rc2 = launch_check("k_rice_decode_vs"))
+    constexpr size_t smem = vc_smem_bytes<32>();
+    if (int rc2 = set_smem(k_rice_decode_vc<16, 32>, smem))
+        return rc2;
+    k_rice_decode_vc<16, 32><<<vs_blocks, 32 * kVsWarps, smem, stream>>>(q, log2s);
+    if (int rc2 = launch_check("k_rice_decode_vc"))
         return rc2;
     DecodeParams pf = p; // whatever was flagged: the general lane-per-stream parser decodes it again
     pf.rice_flags = q.flags;
@@ -911,7 +803,7 @@ static int encode_host(const int16_t *pcm, uint32_t n_frames, uint32_t channels,
     if (n_frames == 0)
         return 0;
     PipelineDrain drain;
-    const ChunkPlan plan = plan_chunks(n_frames, 8, true);
+    const ChunkPlan plan = plan_chunks(n_frames);
     const uint32_t n_chunks = plan.chunks();
     const size_t n_sub = (size_t)n_frames * channels;
     const size_t frame_bytes = (size_t)channels * kFrame * 2;
@@ -995,7 +887,7 @@ static int decode_host(const selab200_subframe_desc *descs, uint32_t n_frames, u
     // Every chunk gets its own compute lane (up to kLanes): the Rice kernel is one lane per stream
     // and latency-bound (about 0.4 ms however small the chunk), so the chunks' Rice kernels must
     // overlap each other and the synthesis kernels of earlier chunks rather than queue up.
-    const ChunkPlan plan = plan_chunks(n_frames, dec_parts(), dec_taper());
+    const ChunkPlan plan = plan_chunks(n_frames);
     const uint32_t n_chunks = plan.chunks();
     const size_t n_sub = (size_t)n_frames * channels;
     const size_t frame_bytes = (size_t)channels * kFrame * 2;
@@ -1465,7 +1357,7 @@ static int container_decode_block(selab200_container *h, uint32_t F0, uint32_t N
     const uint32_t channels = h->info.channels;
     const selab200_subframe_desc *hd = h->buf.h_descs;
     PipelineDrain drain;
-    const ChunkPlan plan = plan_chunks(NF, dec_parts(), dec_taper());
+    const ChunkPlan plan = plan_chunks(NF);
     const uint32_t n_chunks = plan.chunks();
     const size_t n_sub = (size_t)NF * channels;
     const size_t frame_bytes = (size_t)channels * kFrame * 2;

@@ -15,13 +15,14 @@
 //                           the next lane's boundaries are the true ones.  A prefix sum of the
 //                           per-lane symbol counts then names the lane (and, through sparse
 //                           checkpoints, the bit) where symbol t*2048/S begins.
-//   k_rice_decode_vs        one lane per virtual stream, decoding values.
+//   k_rice_decode_vc        one lane per virtual stream, decoding values.
 //
-// Both kernels read the stream the same way: every lane owns a small ring in shared memory that it tops
-// up itself with 16-byte cp.async copies (no cooperation, no registers held across the load latency),
-// and parses from a three-word register window, so that no shared-memory load sits on the
-// symbol-to-symbol dependency chain.  The decoder stages its values in a shared tile and writes them as
-// whole row segments (128-byte lines) instead of one 16-byte store per lane.
+// Both kernels parse from a three-word register window over a small ring in shared memory per lane, so
+// that no shared-memory load sits on the symbol-to-symbol dependency chain.  The split index tops its
+// lane's ring up itself with 16-byte cp.async copies (VsStream); the decoder's rings are topped up by the
+// whole warp in 128-byte segments and bit-reversed in place (VsCoopStream).  The decoder stages its values
+// in a shared tile and writes them as whole row segments (128-byte lines) instead of one 16-byte store per
+// lane.
 //
 // Nothing is taken on trust: part l must end exactly where the table says part l+1 begins (part 0
 // starts at bit 0, so by induction every part is the sequential parse); a stream that fails that
@@ -105,34 +106,6 @@ struct VsRing {
             asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(reinterpret_cast<const char *>(gvec) + (sz ? off : 0u)), "r"(sz) : "memory");
         }
     }
-    // The value parser wants the stream MSB first (a leading-zero count finds the terminator, the payload
-    // reads as a number); the words are reversed once, in place, when their vector has landed -- one BREV per
-    // word instead of one per symbol.  (Behind an inline-asm shared load ptxas lowers BREV to three instructions;
-    // VsCoopStream::reverse_list uses plain loads for that reason.)
-    __device__ __forceinline__ void reverse(uint32_t v) const
-    {
-        const uint32_t a = row | ((16 * v + rot) & kMask);
-        uint32_t x, y, z, w;
-        asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x), "=r"(y), "=r"(z), "=r"(w) : "r"(a));
-        x = __brev(x), y = __brev(y), z = __brev(z), w = __brev(w);
-        asm volatile("st.shared.v4.u32 [%4], {%0, %1, %2, %3};" ::"r"(x), "r"(y), "r"(z), "r"(w), "r"(a) : "memory");
-    }
-    // vectors [lo, hi): two loads in flight before the first BREV
-    __device__ __forceinline__ void reverse_range(uint32_t lo, uint32_t hi) const
-    {
-        for (; lo + 1 < hi; lo += 2) {
-            const uint32_t a = row | ((16 * lo + rot) & kMask), b = row | ((16 * lo + 16 + rot) & kMask);
-            uint32_t x0, y0, z0, w0, x1, y1, z1, w1;
-            asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x0), "=r"(y0), "=r"(z0), "=r"(w0) : "r"(a));
-            asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x1), "=r"(y1), "=r"(z1), "=r"(w1) : "r"(b));
-            x0 = __brev(x0), y0 = __brev(y0), z0 = __brev(z0), w0 = __brev(w0);
-            asm volatile("st.shared.v4.u32 [%4], {%0, %1, %2, %3};" ::"r"(x0), "r"(y0), "r"(z0), "r"(w0), "r"(a) : "memory");
-            x1 = __brev(x1), y1 = __brev(y1), z1 = __brev(z1), w1 = __brev(w1);
-            asm volatile("st.shared.v4.u32 [%4], {%0, %1, %2, %3};" ::"r"(x1), "r"(y1), "r"(z1), "r"(w1), "r"(b) : "memory");
-        }
-        if (lo < hi)
-            reverse(lo);
-    }
 };
 
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
@@ -142,20 +115,20 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // The streaming state of a lane: a window of three words in registers (r0 = word wb - 1 holds the current
 // bit, r1, and r2 loaded one word ahead of its first use) over the ring.  ROUND symbols of at most 32 bits
 // are parsed between two boundaries; at a boundary the ring is topped up as far as the words still needed
-// allow, and the copies issued at the previous boundary are retired (and, for the value parser, reversed).
+// allow, and the copies issued at the previous boundary are retired.
 // A round reads at most ROUND + 2 words past r1.  With RING >= 2 * ROUND + 16 what landed a boundary ago
 // always covers that; a smaller ring (half the shared memory, twice the warps per SM) covers it for
 // ordinary streams and otherwise waits for the copies just issued (RING >= ROUND + 16 suffices then).
-template <int RING, int ROUND, bool REVERSED>
+template <int RING, int ROUND>
 struct VsStream {
     static_assert(RING >= ROUND + 16 && (RING & (RING - 1)) == 0, "ring too small for the round");
     VsRing<RING> rg;
     uint32_t pos;         // current bit, counted from the aligned base
     uint32_t r0, r1, r2;  // window
     uint32_t wa;          // running byte offset (rotated) of r2's word
-    uint32_t fv, rv;      // next vector to request / first vector not yet landed (and reversed)
+    uint32_t fv, rv;      // next vector to request / first vector not yet landed
     uint32_t cv_next;     // vectors below cv_next have been requested by the previous boundary
-    uint32_t ce;          // words below ce have landed (and are reversed)
+    uint32_t ce;          // words below ce have landed
 
     __device__ __forceinline__ uint32_t wb() const { return (pos >> 5) + 1; }
     __device__ __forceinline__ void load_window()
@@ -169,8 +142,6 @@ struct VsStream {
     __device__ __forceinline__ void retire(uint32_t upto) // vectors below `upto` have landed
     {
         if (upto > rv) {
-            if (REVERSED)
-                rg.reverse_range(rv, upto);
             rv = upto;
             ce = 4 * upto;
         }
@@ -229,15 +200,17 @@ struct VsStream {
 
 // ------------------------------------------------------------------ the warp's rings, filled together --
 //
-// The per-lane cp.async of VsStream costs a 16-byte request to 32 different lines per instruction: at scale
-// the load/store unit replays of those requests, not the parse, bound the decoder (measured: the decoder
-// with the top-ups removed runs 2.3x faster).  Here the 32 rings of a warp are topped up COOPERATIVELY in
-// 128-byte segments: a ring is two segments of 32 words; a lane whose parser has left a segment puts its
-// row on a list, and eight lanes copy one row's next segment (8 x 16 bytes = one whole line) -- four rows,
-// four lines per instruction instead of 32 -- and, when it has landed, reverse it the same way.  The copies
-// bypass L1 (cp.async.cg): every line is fetched exactly once, and letting those lines allocate in the 16 KB
-// of L1 the kernel leaves was the second wall (1.43 -> 1.19 ms at 413 k streams).  All calls are
-// warp-convergent.
+// Per-lane cp.async top-ups as in VsStream cost a 16-byte request to 32 different lines per instruction: at
+// scale the load/store unit replays of those requests, not the parse, bound a decoder built that way
+// (measured: with the top-ups removed it ran 2.3x faster).  Here the 32 rings of a warp are topped up
+// COOPERATIVELY in 128-byte segments: a ring is two segments of 32 words; a lane whose parser has left a
+// segment puts its row on a list, and eight lanes copy one row's next segment (8 x 16 bytes = one whole
+// line) -- four rows, four lines per instruction instead of 32 -- and, when it has landed, reverse it the
+// same way.  The value parser wants the stream MSB first (a leading-zero count finds the terminator, the
+// payload reads as a number): reversing each word once, in place, costs one BREV per word instead of one per
+// symbol.  The copies bypass L1 (cp.async.cg): every line is fetched exactly once, and letting those lines
+// allocate in the 16 KB of L1 the kernel leaves was the second wall (1.43 -> 1.19 ms at 413 k streams).  All
+// calls are warp-convergent.
 struct VsCoopMeta { // per warp, in shared memory
     // rows that want a segment, each entry written by the row's owner and read by the eight lanes that copy
     // it (and, a boundary later, reverse it): x, y = source address of the segment; z = bytes of stream left
@@ -260,7 +233,7 @@ __device__ __forceinline__ uint32_t fma_sub(uint32_t a, uint32_t b) // a - b
     return d;
 }
 
-template <int ROUND, bool REVERSED, bool NOCOPY = false>
+template <int ROUND>
 struct VsCoopStream {
     static constexpr int kRing = 64, kSeg = 32;     // words
     static constexpr uint32_t kMask = kRing * 4 - 1;
@@ -337,8 +310,7 @@ struct VsCoopStream {
                 const unsigned long long src = (((unsigned long long)e.y << 32) | e.x) + (sz ? piece : 0u);
                 // the segment may wrap inside the row only at its end: it starts on a 128-byte boundary of the rotated row
                 const uint32_t dst = (e.w & ~kMask) | ((e.w + piece) & kMask);
-                if (!NOCOPY || sz == 77u)
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz) : "memory");
+                asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz) : "memory");
             }
         }
         return n;
@@ -347,21 +319,19 @@ struct VsCoopStream {
     // (all 32 lanes busy -- a lane reversing its own whole segment would leave the other 31 idle).  Convergent.
     __device__ __forceinline__ void reverse_list(int which, int n) const
     {
-        if (REVERSED) {
-            const int lane = lane_id();
-            const uint4 *list = meta->list[which];
-            const uint32_t piece = 16u * (lane & 7);
-            for (int it = 0; it * 4 < n; it++) {
-                const int idx = it * 4 + (lane >> 3);
-                if (idx < n) {
-                    const uint32_t w0 = list[idx].w;
-                    const uint32_t a = (w0 & ~kMask) | ((w0 + piece) & kMask);
-                    // (plain loads through the shared array: behind an inline-asm load ptxas lowers BREV to three instructions)
-                    uint4 *q = reinterpret_cast<uint4 *>(sbase + (a - s0));
-                    uint4 v = *q;
-                    v.x = __brev(v.x), v.y = __brev(v.y), v.z = __brev(v.z), v.w = __brev(v.w);
-                    *q = v;
-                }
+        const int lane = lane_id();
+        const uint4 *list = meta->list[which];
+        const uint32_t piece = 16u * (lane & 7);
+        for (int it = 0; it * 4 < n; it++) {
+            const int idx = it * 4 + (lane >> 3);
+            if (idx < n) {
+                const uint32_t w0 = list[idx].w;
+                const uint32_t a = (w0 & ~kMask) | ((w0 + piece) & kMask);
+                // (plain loads through the shared array: behind an inline-asm load ptxas lowers BREV to three instructions)
+                uint4 *q = reinterpret_cast<uint4 *>(sbase + (a - s0));
+                uint4 v = *q;
+                v.x = __brev(v.x), v.y = __brev(v.y), v.z = __brev(v.z), v.w = __brev(v.w);
+                *q = v;
             }
         }
         __syncwarp(); // reversed words visible to their owners; the list is free again
@@ -494,7 +464,7 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_split_index(RiceVsParams
     const uint32_t total = ok ? (uint32_t)d.res_words + skip : 0u; // words from the aligned base
     const uint32_t k = ok ? d.res_rice_param : 0u, kp1 = k + 1;
 
-    using Stream = VsStream<RING, ROUND, false>;
+    using Stream = VsStream<RING, ROUND>;
     Stream s;
     s.rg.row = smem0 + pad + (uint32_t)(warp * 32 + lane) * (RING * 4);
     s.rg.rot = (16u * lane) & (RING * 4 - 1);
@@ -735,8 +705,8 @@ constexpr size_t split_smem_bytes()
 
 // --------------------------------------------------------------- virtual streams --
 //
-// Geometry (template parameters; the launch picks one):
-//   RING   words per lane in the shared-memory ring
+// k_rice_decode_vc: one lane per virtual stream on the cooperative rings (VsCoopStream, 64 words per lane).
+// Geometry (template parameters; the launch uses ROUND = 16, TILE = 32):
 //   ROUND  symbols a lane decodes between two ring top-ups
 //   TILE   symbols per lane staged in shared memory before they leave as 4*TILE-byte row segments
 
@@ -774,131 +744,6 @@ __device__ __noinline__ bool vs_slow_round(const VsRing<RING> rg, uint32_t ce, u
     return true;
 }
 
-// ABLATE (measurement only, tools/rice_ablation.py; results are wrong): 1 = no global stores, 2 = no ring
-// top-ups after the first fill, 4 = no in-place reversal.
-template <int RING, int ROUND, int TILE, int ABLATE = 0>
-__global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vs(RiceVsParams p, int log2s)
-{
-    static_assert(TILE % ROUND == 0 && TILE % 4 == 0 && ROUND % 4 == 0 && TILE <= 32, "tile geometry");
-    constexpr int kTilePitch = TILE + 4;       // words: rows stay 16-byte aligned, banks rotate by 4 per row
-    constexpr int kRowLanes = TILE / 4;        // lanes that move one row segment (16 bytes each)
-    constexpr int kRowsPerIt = 32 / kRowLanes; // rows per store instruction
-    extern __shared__ __align__(16) unsigned char vs_smem[];
-    const int lane = lane_id(), warp = warp_id();
-    const uint32_t smem0 = (uint32_t)__cvta_generic_to_shared(vs_smem);
-    const uint32_t pad = (RING * 4 - (smem0 & (RING * 4 - 1))) & (RING * 4 - 1);
-    int32_t *tile = reinterpret_cast<int32_t *>(vs_smem + pad + kVsWarps * 32 * RING * 4) + warp * 32 * kTilePitch;
-
-    const uint32_t S = 1u << log2s, part = (uint32_t)kFrame >> log2s;
-    const uint32_t v0 = (blockIdx.x * kVsWarps + warp) * 32;
-    const uint32_t v = v0 + lane, st = v >> log2s, l = v & (S - 1);
-    const bool exists = st < p.n_sub;
-    selab200_subframe_desc d;
-    memset(&d, 0, sizeof d);
-    if (exists)
-        d = p.descs[st];
-    bool ok = exists && rice_desc_ok(d, p.channels, p.n_words);
-    if (exists && !ok && l == 0)
-        raise_status(p.status, SELAB200_ERR_BITSTREAM);
-    const bool store_row = ok; // rows of flagged streams may hold garbage: the general kernel rewrites them
-    uint32_t sb = 0, expect_end = kNoSplit;
-    if (ok && S > 1) {
-        const uint32_t *tb = p.table + (size_t)st * (S - 1);
-        if (tb[0] == kNoSplit) {
-            ok = false; // not split: the general kernel decodes it
-        } else {
-            if (l > 0)
-                sb = tb[l - 1];
-            if (l < S - 1)
-                expect_end = tb[l];
-        }
-    }
-    const uintptr_t addr = reinterpret_cast<uintptr_t>(p.words + (ok ? d.res_offset : 0));
-    const uint32_t skip = (uint32_t)(addr >> 2) & 3u;
-    const uint32_t total = ok && d.res_words ? (uint32_t)d.res_words + skip : 0u;
-    using Stream = VsStream<RING, ROUND, !(ABLATE & 4)>;
-    Stream s;
-    s.rg.row = smem0 + pad + (uint32_t)(warp * 32 + lane) * (RING * 4);
-    s.rg.rot = (16u * lane) & (RING * 4 - 1);
-    s.rg.gvec = reinterpret_cast<const uint4 *>(addr & ~(uintptr_t)15);
-    s.rg.total_bytes = (int)(total * 4);
-    const uint32_t k = ok ? d.res_rice_param : 0u, kp1 = k + 1, kk = 32 - k, kpow = 1u << k;
-    const uint32_t row_mask = __ballot_sync(kFull, store_row);
-
-    uint32_t p0 = sb + 32 * skip;
-    if (p0 > total * 32 + 64)
-        p0 = total * 32 + 64; // a nonsense table entry: parse zeros, fail the end check
-    s.prime(p0);
-    bool dead = false;
-
-    int32_t *out_warp = p.out + (size_t)v0 * part;
-    const uint32_t n_rounds = part / ROUND;
-    const uint32_t c_pn = kp1 + 31;
-#pragma unroll 1
-    for (uint32_t r = 0; r < n_rounds; r++) {
-        if (r && !dead && !(ABLATE & 2))
-            s.boundary();
-        uint32_t pos_s = s.pos;
-        int mn = 31; // lowest FLO result of the round; below k: a symbol longer than the window
-        int32_t *trow = tile + lane * kTilePitch + (r % (TILE / ROUND)) * ROUND;
-#pragma unroll
-        for (int e4 = 0; e4 < ROUND; e4 += 4) {
-            int32_t val[4];
-#pragma unroll
-            for (int e = 0; e < 4; e++) {
-                const uint32_t win = __funnelshift_l(s.r1, s.r0, s.pos);
-                const uint32_t f = bfind_u32(~win);   // 31 - ones; 0xffffffff: the window is all ones
-                const uint32_t pn = s.pos + c_pn - f; // pos + ones + 1 + k
-                mn = min(mn, (int)f);
-                const uint32_t ones = 31 - f;
-                const uint32_t t = __funnelshift_lc(0u, win, ones + 1);
-                const uint32_t pay = __funnelshift_rc(t, 0u, kk);
-                val[e] = unzigzag3(ones * kpow + pay);
-                if ((s.pos ^ pn) >= 32u)
-                    s.advance();
-                s.pos = pn;
-            }
-            *reinterpret_cast<int4 *>(trow + e4) = make_int4(val[0], val[1], val[2], val[3]);
-        }
-        if (mn < (int)k && !dead && !(ABLATE & 6)) { // a symbol longer than the window: redo the round with the general parser
-            if (vs_slow_round<RING>(s.rg, s.ce, &pos_s, k, trow, ROUND)) {
-                s.pos = pos_s;
-                s.load_window();
-            } else {
-                dead = true;
-            }
-        }
-        // ---- a full tile: TILE symbols per lane leave as row segments of 4*TILE bytes ----
-        if (r % (TILE / ROUND) == TILE / ROUND - 1) {
-            __syncwarp();
-            int32_t *dst = out_warp + (size_t)(r / (TILE / ROUND)) * TILE + (lane % kRowLanes) * 4;
-#pragma unroll
-            for (int it = 0; it < 32 / kRowsPerIt; it++) {
-                const int row = kRowsPerIt * it + lane / kRowLanes;
-                if ((row_mask >> row) & 1u) {
-                    const int4 q = *reinterpret_cast<const int4 *>(tile + row * kTilePitch + (lane % kRowLanes) * 4);
-                    if (!(ABLATE & 1) || q.x == 0x7fffffff)
-                        *reinterpret_cast<int4 *>(dst + (size_t)row * part) = q;
-                }
-            }
-            __syncwarp();
-        }
-    }
-    cp_async_wait<0>();
-    if (exists && store_row) {
-        bool bad = dead;
-        if (ok) {
-            if (expect_end != kNoSplit)
-                bad |= s.pos - 32 * skip != expect_end;
-            else
-                bad |= s.pos > total * 32;
-        }
-        if (bad && !(ABLATE & 6))
-            p.flags[st] = 1u; // (several parts may say so: idempotent)
-    }
-}
-
-// The decoder on the cooperative rings (VsCoopStream): same parse, same tile, warp-wide top-ups.
 template <int RING>
 __device__ __noinline__ bool vc_slow_round(uint32_t row, uint32_t rot, uint32_t ce, uint32_t *pos, uint32_t k, int32_t *dst, int count)
 {
@@ -910,15 +755,15 @@ __device__ __noinline__ bool vc_slow_round(uint32_t row, uint32_t rot, uint32_t 
     return vs_slow_round<RING>(rg, ce, pos, k, dst, count);
 }
 
-template <int ROUND, int TILE, int ABLATE = 0>
+template <int ROUND, int TILE>
 __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p, int log2s)
 {
-    using Stream = VsCoopStream<ROUND, !(ABLATE & 4), (ABLATE & 8) != 0>;
+    using Stream = VsCoopStream<ROUND>;
     constexpr int RING = Stream::kRing;
     static_assert(TILE % ROUND == 0 && TILE % 4 == 0 && ROUND % 4 == 0 && TILE <= 128, "tile geometry");
-    constexpr int kTilePitch = TILE + 4;
-    constexpr int kRowLanes = TILE / 4;
-    constexpr int kRowsPerIt = 32 / kRowLanes;
+    constexpr int kTilePitch = TILE + 4;       // words: rows stay 16-byte aligned, banks rotate by 4 per row
+    constexpr int kRowLanes = TILE / 4;        // lanes that move one row segment (16 bytes each)
+    constexpr int kRowsPerIt = 32 / kRowLanes; // rows per store instruction
     extern __shared__ __align__(16) unsigned char vc_smem[];
     const int lane = lane_id(), warp = warp_id();
     const uint32_t smem0 = (uint32_t)__cvta_generic_to_shared(vc_smem);
@@ -969,7 +814,7 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p
     const uint32_t c_pn = kp1 + 31;
 #pragma unroll 1
     for (uint32_t r = 0; r < n_rounds; r++) {
-        if (r && !(ABLATE & 2))
+        if (r)
             s.boundary(!dead);
         uint32_t pos_s = s.pos;
         int mn = 31; // lowest FLO result of the round; below k: a symbol longer than the window
@@ -993,7 +838,7 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p
             }
             *reinterpret_cast<int4 *>(trow + e4) = make_int4(val[0], val[1], val[2], val[3]);
         }
-        if (mn < (int)k && !dead && !(ABLATE & 14)) { // a symbol longer than the window: redo the round with the general parser
+        if (mn < (int)k && !dead) { // a symbol longer than the window: redo the round with the general parser
             if (vc_slow_round<RING>(s.row, s.rot, s.ce, &pos_s, k, trow, ROUND)) {
                 s.pos = pos_s;
                 s.load_window();
@@ -1003,6 +848,7 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p
         }
         if (dead)
             s.pos = pos_s; // parked: its ring is not topped up any more
+        // ---- a full tile: TILE symbols per lane leave as row segments of 4*TILE bytes ----
         if (r % (TILE / ROUND) == TILE / ROUND - 1) {
             __syncwarp();
             int32_t *dst = out_warp + (size_t)(r / (TILE / ROUND)) * TILE + (lane % kRowLanes) * 4;
@@ -1011,12 +857,7 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p
                 const int row = kRowsPerIt * it + lane / kRowLanes;
                 if ((row_mask >> row) & 1u) {
                     const int4 q = *reinterpret_cast<const int4 *>(tile + row * kTilePitch + (lane % kRowLanes) * 4);
-                    if (!(ABLATE & 1) || q.x == 0x7fffffff) {
-                        if (ABLATE & 16)
-                            __stcs(reinterpret_cast<int4 *>(dst + (size_t)row * part), q);
-                        else
-                            *reinterpret_cast<int4 *>(dst + (size_t)row * part) = q;
-                    }
+                    *reinterpret_cast<int4 *>(dst + (size_t)row * part) = q;
                 }
             }
             __syncwarp();
@@ -1031,8 +872,8 @@ __global__ void __launch_bounds__(32 * kVsWarps) k_rice_decode_vc(RiceVsParams p
             else
                 bad |= s.pos > total * 32;
         }
-        if (bad && !(ABLATE & 14))
-            p.flags[st] = 1u;
+        if (bad)
+            p.flags[st] = 1u; // (several parts may say so: idempotent)
     }
 }
 
@@ -1040,12 +881,6 @@ template <int TILE>
 constexpr size_t vc_smem_bytes()
 {
     return 64 * 4 + (size_t)kVsWarps * 32 * 64 * 4 + (size_t)kVsWarps * 32 * (TILE + 4) * 4 + kVsWarps * sizeof(VsCoopMeta);
-}
-
-template <int RING, int TILE>
-constexpr size_t vs_smem_bytes()
-{
-    return RING * 4 + (size_t)kVsWarps * 32 * RING * 4 + (size_t)kVsWarps * 32 * (TILE + 4) * 4;
 }
 
 } // namespace selab200

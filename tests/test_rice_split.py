@@ -1,5 +1,5 @@
 """GPU parity of the second-generation Rice decoder (sela_b200/csrc/rice_vs.cuh): streams cut into S parts
-by k_rice_split_index and decoded by k_rice_decode_vs, for every S, against the reference's decoder
+by k_rice_split_index and decoded by k_rice_decode_vc, for every S, against the reference's decoder
 (rice::RiceDecoder, src/rice/rice_decoder.cpp:11-52) -- including the streams it must hand back to the
 general parser (periodic streams that never resynchronise, long unary runs, streams with more symbols per part than it keeps checkpoints for)."""
 import numpy as np

@@ -2,7 +2,7 @@
 
 north_star asks for ">= 70 % of HBM roofline on the Rice decode kernel".  The kernel is one lane per
 stream; at BASELINE's batch (25 838 streams = 808 warps) it is starved for parallelism.  This sweeps
-the number of streams by tiling the coded 10-minute stereo file, and both ring geometries.
+the number of streams by tiling the coded 10-minute stereo file.
 Algorithmic bytes (SURVEY.md 8d): residue words read + 4 B per decoded sample written.
 Run on the GPU box:  python tools/rice_decode_roofline.py [max_tile]
 """
@@ -62,7 +62,7 @@ for tile in [t for t in TILES if t <= max_tile]:
         for _ in range(args.warm):
             run()
         torch.cuda.synchronize()
-        assert int(status.item()) == 0 or os.environ.get("SELAB200_RICE_GEOM", "0") >= "100"
+        assert int(status.item()) == 0
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
         reps = args.reps
         ev[0].record()
