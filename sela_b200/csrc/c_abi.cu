@@ -39,33 +39,60 @@ int fail(int code, const char *fmt, ...)
             return fail(SELAB200_ERR_CUDA, "%s failed: %s", #expr, cudaGetErrorString(e_)); \
     } while (0)
 
-struct DeviceBuffer {
+// A grow-only allocation, on the device or pinned on the host: a request that fits keeps the block, a
+// larger one replaces it with an eighth plus 4 KB to spare.
+template <bool Pinned>
+struct GrowBuffer {
     void *ptr = nullptr;
     size_t bytes = 0;
     int ensure(size_t need)
     {
         if (need <= bytes)
             return 0;
-        if (ptr)
-            cudaFree(ptr);
-        ptr = nullptr;
-        bytes = 0;
-        size_t want = need + need / 8 + 4096;
-        cudaError_t e = cudaMalloc(&ptr, want);
+        release();
+        const size_t want = need + need / 8 + 4096;
+        const cudaError_t e = Pinned ? cudaMallocHost(&ptr, want) : cudaMalloc(&ptr, want);
         if (e != cudaSuccess)
-            return fail(SELAB200_ERR_CUDA, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+            return Pinned ? fail(SELAB200_ERR_CUDA, "cudaMallocHost(%zu) failed", want)
+                          : fail(SELAB200_ERR_CUDA, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
         bytes = want;
         return 0;
     }
     void release()
     {
-        if (ptr)
+        if (ptr && Pinned)
+            cudaFreeHost(ptr);
+        else if (ptr)
             cudaFree(ptr);
         ptr = nullptr;
         bytes = 0;
     }
 };
+using DeviceBuffer = GrowBuffer<false>;
+using PinnedBuffer = GrowBuffer<true>;
 
+// What a container handle owns besides the walk result: the device image of the bytes, a pinned
+// descriptor table and the upload events.  Recycled through a small free list, because a process
+// that decodes many files would otherwise pay cudaMalloc/cudaFree (a device-wide sync) and
+// cudaMallocHost/cudaFreeHost for every one of them.
+struct ContainerBuffers {
+    static constexpr int kPieces = 8;
+    DeviceBuffer image;
+    PinnedBuffer descs; // selab200_subframe_desc, file order
+    cudaEvent_t ev_piece[kPieces] = {};
+    void destroy()
+    {
+        for (cudaEvent_t &e : ev_piece)
+            if (e) {
+                cudaEventDestroy(e);
+                e = nullptr;
+            }
+        image.release();
+        descs.release();
+    }
+};
+
+constexpr size_t kMaxSpareBuffers = 16;
 constexpr int kMaxChunks = 72;
 constexpr int kLanes = 8; // concurrent compute streams of the pipelined host calls
 
@@ -82,65 +109,59 @@ struct Context {
     unsigned long long *h_totals = nullptr;        // pinned: arena fill level after each chunk
     size_t last_rice_n_sub = 0;                    // selab200_rice_decode_frames_device bookkeeping (flag count query)
     cudaStream_t last_rice_stream = nullptr;
-    std::vector<struct ContainerBuffers> *spare = nullptr; // recycled container buffers of this device
+    std::vector<ContainerBuffers> spare;           // recycled container buffers of this device (g_mutex held)
 };
 
 // One context per device the library was initialised for (selab200_init / selab200_init_devices), slot 0 the
-// primary.  Everything below reaches "the" context through `g`, a thread-local pointer: an API call runs on
-// the primary (or, for the *_device forms, on the device that owns the caller's pointers); the multi-device
-// host-buffer calls give every device a worker thread of its own that points `g` at that device's context.
-// Contexts share nothing, so the workers never contend.
+// primary.  An API call runs on the primary (or, for the *_device forms, on the device that owns the caller's
+// pointers) and hands that context down; the multi-device host-buffer calls give every device a worker thread
+// of its own, with that device's context.  Contexts share nothing, so the workers never contend.
 constexpr int kMaxDevices = 16;
 Context g_slots[kMaxDevices];
 int g_n_ctx = 0;
-Context *g_last_rice_ctx = nullptr; // the context selab200_rice_decode_frames_device last ran on (flag count query)
-thread_local Context *tl_ctx = &g_slots[0];
-#define g (*tl_ctx)
+int g_last_rice_slot = -1; // the slot selab200_rice_decode_frames_device last ran on (flag count query)
 
-// What a container handle owns besides the walk result: the device image of the bytes, a pinned
-// descriptor table and the upload events.  Recycled through a small free list, because a process
-// that decodes many files would otherwise pay cudaMalloc/cudaFree (a device-wide sync) and
-// cudaMallocHost/cudaFreeHost for every one of them.
-struct ContainerBuffers {
-    static constexpr int kPieces = 8;
-    void *d_bytes = nullptr;
-    size_t d_cap = 0;
-    selab200_subframe_desc *h_descs = nullptr;
-    size_t h_cap = 0; // descriptors
-    cudaEvent_t ev_piece[kPieces] = {};
-    void destroy()
-    {
-        for (cudaEvent_t &e : ev_piece)
-            if (e) {
-                cudaEventDestroy(e);
-                e = nullptr;
-            }
-        if (d_bytes)
-            cudaFree(d_bytes);
-        if (h_descs)
-            cudaFreeHost(h_descs);
-        d_bytes = nullptr;
-        h_descs = nullptr;
-        d_cap = h_cap = 0;
-    }
-};
+// Makes the context's device the calling thread's current one: the current device is per host thread, and
+// callers may arrive on a thread other than init()'s.
+int use_device(const Context &c)
+{
+    cudaError_t e = cudaSetDevice(c.device);
+    if (e != cudaSuccess)
+        return fail(SELAB200_ERR_CUDA, "cudaSetDevice(%d) failed: %s", c.device, cudaGetErrorString(e));
+    return 0;
+}
 
-std::vector<ContainerBuffers> g_spare_store[kMaxDevices]; // guarded by g_mutex; Context::spare points here
-#define g_spare_buffers (*g.spare)
-constexpr size_t kMaxSpareBuffers = 16;
+// Returns `rc` after `cleanup`, keeping the message of the error that caused it.
+template <typename F>
+int fail_after_cleanup(int rc, F cleanup)
+{
+    char keep[sizeof g_error];
+    memcpy(keep, g_error, sizeof keep);
+    cleanup();
+    memcpy(g_error, keep, sizeof keep);
+    return rc;
+}
+
+int check_channels(uint32_t channels)
+{
+    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
+        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    return 0;
+}
 
 // On every exit from a pipelined call -- error paths included -- nothing may still be
 // reading or writing the caller's host buffers.
 struct PipelineDrain {
+    Context &c;
     ~PipelineDrain()
     {
-        if (g.s_h2d)
-            cudaStreamSynchronize(g.s_h2d);
+        if (c.s_h2d)
+            cudaStreamSynchronize(c.s_h2d);
         for (int i = 0; i < kLanes; i++)
-            if (g.s_compute[i])
-                cudaStreamSynchronize(g.s_compute[i]);
-        if (g.s_d2h)
-            cudaStreamSynchronize(g.s_d2h);
+            if (c.s_compute[i])
+                cudaStreamSynchronize(c.s_compute[i]);
+        if (c.s_d2h)
+            cudaStreamSynchronize(c.s_d2h);
     }
 };
 
@@ -198,24 +219,21 @@ const char *status_text(int s)
     }
 }
 
-// Points `g` at the primary context for the calling thread (g_mutex held) and selects its device.
-int require_ready()
+// Sets `c` to the primary context and makes its device current (g_mutex held).
+int require_ready(Context *&c)
 {
-    tl_ctx = &g_slots[0];
-    if (g_n_ctx == 0 || !g.ready)
+    c = &g_slots[0];
+    if (g_n_ctx == 0 || !c->ready)
         return fail(SELAB200_ERR_NOT_INIT, "selab200_init() has not been called (or found no CUDA device)");
-    // the current device is per host thread; callers may arrive on a thread other than init()'s
-    cudaError_t e = cudaSetDevice(g.device);
-    if (e != cudaSuccess)
-        return fail(SELAB200_ERR_CUDA, "cudaSetDevice(%d) failed: %s", g.device, cudaGetErrorString(e));
-    return 0;
+    return use_device(*c);
 }
 
-// The *_device forms run on the device that owns the caller's buffers: points `g` at that device's context.
-int require_ready_for(const void *device_ptr)
+// The *_device forms run on the device that owns the caller's buffers: sets `c` to that device's context and
+// makes it current.  A null pointer selects the primary (the caller reports the null pointer).
+int require_ready_for(const void *device_ptr, Context *&c)
 {
-    if (g_n_ctx == 0)
-        return require_ready();
+    if (!device_ptr || g_n_ctx == 0)
+        return require_ready(c);
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, device_ptr) != cudaSuccess || attr.type != cudaMemoryTypeDevice) {
         cudaGetLastError();
@@ -223,11 +241,8 @@ int require_ready_for(const void *device_ptr)
     }
     for (int i = 0; i < g_n_ctx; i++)
         if (g_slots[i].ready && g_slots[i].device == attr.device) {
-            tl_ctx = &g_slots[i];
-            cudaError_t e = cudaSetDevice(g.device);
-            if (e != cudaSuccess)
-                return fail(SELAB200_ERR_CUDA, "cudaSetDevice(%d) failed: %s", g.device, cudaGetErrorString(e));
-            return 0;
+            c = &g_slots[i];
+            return use_device(*c);
         }
     return fail(SELAB200_ERR_ARGUMENT, "the buffers live on device %d, which the library was not initialised for "
                                        "(selab200_init / selab200_init_devices)", attr.device);
@@ -279,8 +294,8 @@ int encode_device(const int16_t *d_pcm, uint32_t n_frames, uint32_t channels, se
                   cudaEvent_t after_scan = nullptr, unsigned long long *h_fill_after = nullptr,
                   uint8_t *d_container = nullptr, unsigned long long sub_base = 0)
 {
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     if (ws_bytes < selab200_encode_workspace_bytes(n_frames, channels))
         return fail(SELAB200_ERR_ARGUMENT, "encode workspace too small");
     if (channels == 2 && (reinterpret_cast<uintptr_t>(d_pcm) & 15) != 0) // the stereo kernel reads 16 bytes (4 sample pairs) at a time
@@ -430,12 +445,26 @@ int launch_rice_residues(const DecodeParams &p, void *aux, cudaStream_t stream)
     return launch_rice_decode(pf, 1, stream);
 }
 
+// The inputs every decode kernel reads; the workspace and output pointers are left null for the caller.
+DecodeParams decode_params(const selab200_subframe_desc *d_descs, uint32_t n_frames, uint32_t channels,
+                           const uint32_t *d_words, size_t n_words, int32_t *d_status)
+{
+    DecodeParams p = {};
+    p.descs = d_descs;
+    p.n_frames = n_frames;
+    p.channels = channels;
+    p.words = d_words;
+    p.n_words = n_words;
+    p.status = d_status;
+    return p;
+}
+
 int decode_device(const selab200_subframe_desc *d_descs, uint32_t n_frames, uint32_t channels,
                   const uint32_t *d_words, size_t n_words, int16_t *d_pcm, int32_t *d_status, void *d_ws,
                   size_t ws_bytes, cudaStream_t stream, bool fresh = true)
 {
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     if (ws_bytes < selab200_decode_workspace_bytes(n_frames, channels))
         return fail(SELAB200_ERR_ARGUMENT, "decode workspace too small");
     if (fresh)
@@ -443,18 +472,11 @@ int decode_device(const selab200_subframe_desc *d_descs, uint32_t n_frames, uint
     if (n_frames == 0)
         return 0;
     const size_t n_sub = (size_t)n_frames * channels;
-    DecodeParams p;
-    p.descs = d_descs;
-    p.n_frames = n_frames;
-    p.channels = channels;
-    p.words = d_words;
-    p.n_words = n_words;
+    DecodeParams p = decode_params(d_descs, n_frames, channels, d_words, n_words, d_status);
     p.pcm_out = d_pcm;
-    p.status = d_status;
     p.ws_q = static_cast<int32_t *>(d_ws);
     p.ws_res = reinterpret_cast<int32_t *>(static_cast<char *>(d_ws) + align256(n_sub * 128 * 4));
     p.order_index = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(p.ws_res) + align256(n_sub * kFrame * 4));
-    p.rice_flags = nullptr;
     void *rice_aux = reinterpret_cast<char *>(p.order_index) + align256((n_sub + 16) * 4);
     const size_t n_slots = (n_sub + 12 + 3) / 4 * 4; // every class segment starts on a warp boundary
     CUDA_TRY(cudaMemsetAsync(p.order_index, 0xff, n_slots * 4, stream));
@@ -484,12 +506,12 @@ int decode_device(const selab200_subframe_desc *d_descs, uint32_t n_frames, uint
     return launch_check("k_synthesise");
 }
 
-int read_status(cudaStream_t stream, const int32_t *d_status)
+int read_status(Context &c, cudaStream_t stream, const int32_t *d_status)
 {
-    CUDA_TRY(cudaMemcpyAsync(g.h_small, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemcpyAsync(c.h_small, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
-    if (g.h_small[0] != 0)
-        return fail(g.h_small[0], "%s", status_text(g.h_small[0]));
+    if (c.h_small[0] != 0)
+        return fail(c.h_small[0], "%s", status_text(c.h_small[0]));
     return 0;
 }
 
@@ -501,8 +523,8 @@ int selab200_abi_version(void) { return SELAB200_ABI_VERSION; }
 const char *selab200_last_error(void) { return g_error; }
 uint64_t selab200_launch_count(void) { return g_launches.load(); }
 
-// (g_mutex held; `g` points at the slot to set up)
-static int init_slot(int device, int slot)
+// (g_mutex held)
+static int init_slot(Context &c, int device)
 {
     CUDA_TRY(cudaSetDevice(device));
     cudaDeviceProp prop;
@@ -510,86 +532,71 @@ static int init_slot(int device, int slot)
     if (prop.major < 10)
         return fail(SELAB200_ERR_NO_DEVICE, "device %d is sm_%d%d; this build targets sm_100a only", device,
                     prop.major, prop.minor);
-    CUDA_TRY(cudaStreamCreateWithFlags(&g.stream, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamCreateWithFlags(&g.s_h2d, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamCreateWithFlags(&g.s_d2h, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&c.s_h2d, cudaStreamNonBlocking));
+    CUDA_TRY(cudaStreamCreateWithFlags(&c.s_d2h, cudaStreamNonBlocking));
     for (int i = 0; i < kLanes; i++)
-        CUDA_TRY(cudaStreamCreateWithFlags(&g.s_compute[i], cudaStreamNonBlocking));
+        CUDA_TRY(cudaStreamCreateWithFlags(&c.s_compute[i], cudaStreamNonBlocking));
     for (int i = 0; i < kMaxChunks; i++) {
-        CUDA_TRY(cudaEventCreateWithFlags(&g.ev_h2d[i], cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&g.ev_done[i], cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&g.ev_scan[i], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&c.ev_h2d[i], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&c.ev_done[i], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&c.ev_scan[i], cudaEventDisableTiming));
     }
-    CUDA_TRY(cudaEventCreateWithFlags(&g.ev_reset, cudaEventDisableTiming));
-    g.events = true;
-    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&g.h_small), 64));
-    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&g.h_totals), (kMaxChunks + 1) * 8));
-    if (int rc = g.small.ensure(256))
+    CUDA_TRY(cudaEventCreateWithFlags(&c.ev_reset, cudaEventDisableTiming));
+    c.events = true;
+    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&c.h_small), 64));
+    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&c.h_totals), (kMaxChunks + 1) * 8));
+    if (int rc = c.small.ensure(256))
         return rc;
-    g.spare = &g_spare_store[slot];
-    g.device = device;
-    g.ready = true;
+    c.device = device;
+    c.ready = true;
     return 0;
 }
 
-static void shutdown_slot()
+static void shutdown_slot(Context &c)
 {
-    if (g.device >= 0)
-        cudaSetDevice(g.device);
-    if (g.stream)
-        cudaStreamSynchronize(g.stream);
-    if (g.spare) {
-        for (ContainerBuffers &b : *g.spare)
-            b.destroy();
-        g.spare->clear();
-    }
-    g.in.release();
-    g.descs.release();
-    g.words.release();
-    g.work.release();
+    if (c.device >= 0)
+        cudaSetDevice(c.device);
+    if (c.stream)
+        cudaStreamSynchronize(c.stream);
+    for (ContainerBuffers &b : c.spare)
+        b.destroy();
+    c.spare.clear();
+    c.in.release();
+    c.descs.release();
+    c.words.release();
+    c.work.release();
     for (int i = 0; i < kLanes; i++)
-        g.lane_work[i].release();
-    g.aux.release();
-    g.small.release();
-    if (g.h_small)
-        cudaFreeHost(g.h_small);
-    g.h_small = nullptr;
-    if (g.h_totals)
-        cudaFreeHost(g.h_totals);
-    g.h_totals = nullptr;
-    for (cudaStream_t st : {g.stream, g.s_h2d, g.s_d2h})
+        c.lane_work[i].release();
+    c.aux.release();
+    c.small.release();
+    if (c.h_small)
+        cudaFreeHost(c.h_small);
+    if (c.h_totals)
+        cudaFreeHost(c.h_totals);
+    for (cudaStream_t st : {c.stream, c.s_h2d, c.s_d2h})
         if (st)
             cudaStreamDestroy(st);
-    for (int i = 0; i < kLanes; i++) {
-        if (g.s_compute[i])
-            cudaStreamDestroy(g.s_compute[i]);
-        g.s_compute[i] = nullptr;
-    }
-    g.stream = g.s_h2d = g.s_d2h = nullptr;
-    if (g.events) {
+    for (int i = 0; i < kLanes; i++)
+        if (c.s_compute[i])
+            cudaStreamDestroy(c.s_compute[i]);
+    if (c.events) {
         for (int i = 0; i < kMaxChunks; i++) {
-            cudaEventDestroy(g.ev_h2d[i]);
-            cudaEventDestroy(g.ev_done[i]);
-            cudaEventDestroy(g.ev_scan[i]);
+            cudaEventDestroy(c.ev_h2d[i]);
+            cudaEventDestroy(c.ev_done[i]);
+            cudaEventDestroy(c.ev_scan[i]);
         }
-        cudaEventDestroy(g.ev_reset);
+        cudaEventDestroy(c.ev_reset);
     }
-    g.events = false;
-    g.ready = false;
-    g.device = -1;
-    g.last_rice_n_sub = 0;
-    if (g_last_rice_ctx == tl_ctx)
-        g_last_rice_ctx = nullptr;
+    c = Context(); // not ready, no device, every handle null
 }
 
 static void shutdown_all()
 {
-    for (int i = 0; i < g_n_ctx; i++) {
-        tl_ctx = &g_slots[i];
-        shutdown_slot();
-    }
+    for (int i = 0; i < g_n_ctx; i++)
+        shutdown_slot(g_slots[i]);
     g_n_ctx = 0;
-    tl_ctx = &g_slots[0];
+    g_last_rice_slot = -1;
 }
 
 int selab200_init_devices(int count, const int *devices)
@@ -600,10 +607,8 @@ int selab200_init_devices(int count, const int *devices)
     bool same = count == g_n_ctx;
     for (int i = 0; same && i < count; i++)
         same = g_slots[i].ready && g_slots[i].device == devices[i];
-    if (same) {
-        tl_ctx = &g_slots[0];
+    if (same)
         return 0;
-    }
     int have = 0;
     cudaError_t e = cudaGetDeviceCount(&have);
     if (e != cudaSuccess || have == 0)
@@ -619,19 +624,12 @@ int selab200_init_devices(int count, const int *devices)
     // a different set of devices than before: everything the old contexts own (streams, events, pools) lives on
     // the old devices, so they are torn down completely before the new ones are set up
     shutdown_all();
-    for (int i = 0; i < count; i++) {
-        tl_ctx = &g_slots[i];
-        if (int rc = init_slot(devices[i], i)) {
-            char keep[sizeof g_error];
-            memcpy(keep, g_error, sizeof keep);
+    for (int i = 0; i < count; i++)
+        if (int rc = init_slot(g_slots[i], devices[i])) {
             g_n_ctx = i + 1;
-            shutdown_all();
-            memcpy(g_error, keep, sizeof keep);
-            return rc;
+            return fail_after_cleanup(rc, shutdown_all);
         }
-    }
     g_n_ctx = count;
-    tl_ctx = &g_slots[0];
     CUDA_TRY(cudaSetDevice(g_slots[0].device));
     return 0;
 }
@@ -692,7 +690,8 @@ int selab200_encode_frames_device(const int16_t *d_pcm, uint32_t n_frames, uint3
                                   size_t workspace_bytes, void *stream)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = d_pcm ? require_ready_for(d_pcm) : require_ready())
+    Context *c;
+    if (int rc = require_ready_for(d_pcm, c))
         return rc;
     if (!d_pcm || !d_descs || !d_words || !d_words_used || !d_status || !d_workspace)
         return fail(SELAB200_ERR_ARGUMENT, "null device pointer");
@@ -705,7 +704,8 @@ int selab200_decode_frames_device(const selab200_subframe_desc *d_descs, uint32_
                                   void *d_workspace, size_t workspace_bytes, void *stream)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = d_descs ? require_ready_for(d_descs) : require_ready())
+    Context *c;
+    if (int rc = require_ready_for(d_descs, c))
         return rc;
     if (!d_descs || !d_words || !d_pcm_out || !d_status || !d_workspace)
         return fail(SELAB200_ERR_ARGUMENT, "null device pointer");
@@ -713,71 +713,55 @@ int selab200_decode_frames_device(const selab200_subframe_desc *d_descs, uint32_
                          workspace_bytes, (cudaStream_t)stream);
 }
 
-// Host-buffer batch calls.  Pipelined in chunks of frames over three engines:
-//   s_h2d      PCM (encode) / descriptors + words (decode) of chunk c+1 .. go up
-//   s_compute  two alternating lanes run the kernels of chunk c (tails of one chunk overlap the
-//              head of the next; the encoder's scans are chained by events because each needs
-//              the arena fill level its predecessor left in *d_used)
-//   s_d2h      results of chunk c-1 come down
-// With pinned host buffers (selab200_host_alloc) the three overlap; pageable memory works
-// but serialises inside the driver.
 int selab200_rice_decode_frames_device(const selab200_subframe_desc *d_descs, uint32_t n_frames, uint32_t channels,
                                        const uint32_t *d_words, size_t n_words, int32_t *d_residues,
                                        int32_t *d_status, void *stream)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = d_descs ? require_ready_for(d_descs) : require_ready())
+    Context *c;
+    if (int rc = require_ready_for(d_descs, c))
         return rc;
     if (!d_descs || !d_words || !d_residues || !d_status)
         return fail(SELAB200_ERR_ARGUMENT, "null device pointer");
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int32_t), (cudaStream_t)stream));
     if (n_frames == 0)
         return 0;
-    DecodeParams p;
-    p.descs = d_descs;
-    p.n_frames = n_frames;
-    p.channels = channels;
-    p.words = d_words;
-    p.n_words = n_words;
-    p.pcm_out = nullptr;
-    p.status = d_status;
-    p.ws_q = nullptr;
+    DecodeParams p = decode_params(d_descs, n_frames, channels, d_words, n_words, d_status);
     p.ws_res = d_residues;
-    p.order_index = nullptr;
-    p.fallback_only = 0;
-    p.rice_flags = nullptr;
-    if (int rc = g.aux.ensure((size_t)n_frames * channels * 64 + 256))
+    if (int rc = c->aux.ensure((size_t)n_frames * channels * 64 + 256))
         return rc;
-    g.last_rice_n_sub = (size_t)n_frames * channels;
-    g.last_rice_stream = (cudaStream_t)stream;
-    g_last_rice_ctx = tl_ctx;
-    return launch_rice_residues(p, g.aux.ptr, (cudaStream_t)stream);
+    c->last_rice_n_sub = (size_t)n_frames * channels;
+    c->last_rice_stream = (cudaStream_t)stream;
+    g_last_rice_slot = (int)(c - g_slots);
+    return launch_rice_residues(p, c->aux.ptr, (cudaStream_t)stream);
 }
 
 int selab200_rice_decode_flagged(uint32_t *n_flagged)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!n_flagged)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
     *n_flagged = 0;
-    if (g_last_rice_ctx && g_last_rice_ctx->ready) { // the device the last call ran on, which need not be the primary
-        tl_ctx = g_last_rice_ctx;
-        CUDA_TRY(cudaSetDevice(g.device));
+    if (g_last_rice_slot >= 0 && g_slots[g_last_rice_slot].ready) { // the device the last call ran on, which need not be the primary
+        c = &g_slots[g_last_rice_slot];
+        if (int rc = use_device(*c))
+            return rc;
     }
-    const size_t n = g.last_rice_n_sub;
-    if (n == 0 || g.aux.bytes < n * 64)
+    const size_t n = c->last_rice_n_sub;
+    if (n == 0 || c->aux.bytes < n * 64)
         return 0;
     std::vector<uint32_t> flags(n);
-    CUDA_TRY(cudaStreamSynchronize(g.last_rice_stream));
-    CUDA_TRY(cudaMemcpy(flags.data(), static_cast<uint32_t *>(g.aux.ptr) + n * 15, n * 4, cudaMemcpyDeviceToHost));
-    uint32_t c = 0;
+    CUDA_TRY(cudaStreamSynchronize(c->last_rice_stream));
+    CUDA_TRY(cudaMemcpy(flags.data(), static_cast<uint32_t *>(c->aux.ptr) + n * 15, n * 4, cudaMemcpyDeviceToHost));
+    uint32_t count = 0;
     for (uint32_t f : flags)
-        c += f != 0;
-    *n_flagged = c;
+        count += f != 0;
+    *n_flagged = count;
     return 0;
 }
 
@@ -789,125 +773,166 @@ static unsigned long long container_frame_byte(unsigned long long f, uint32_t ch
     return kContainerHeaderBytes + 4 * f + (unsigned long long)kSubframeHeaderBytes * f * channels + 4 * words;
 }
 
+// ---- pipelined host-buffer calls ----------------------------------------------------------------
+//
+// Encode, decode and container decode run in chunks of frames (plan_chunks) over three engines:
+//   s_h2d      PCM (encode) / descriptors + words (decode) of chunk c+1 .. go up
+//   s_compute  the compute lanes run the kernels of chunk c (tails of one chunk overlap the head of
+//              the next); encode alternates two lanes whose scans are chained by events, because each
+//              needs the arena fill level its predecessor left in *d_used
+//   s_d2h      results of chunk c-1 come down
+// With pinned host buffers (selab200_host_alloc) the three overlap; pageable memory works
+// but serialises inside the driver.
+
+// Device views of a pipelined call's buffers.
+struct PipelineViews {
+    int32_t *status;               // Context::small, bytes 0..3
+    uint64_t *used;                // Context::small, bytes 8..15: arena fill level (encode)
+    int16_t *pcm;                  // Context::in
+    selab200_subframe_desc *descs; // Context::descs
+    uint32_t *words;               // Context::words
+};
+
+// The start every pipelined call shares: grows the context's buffers for the frames of `plan` (`words_bytes` of
+// word arena or container image, `ws_bytes` of workspace on each of the first `lanes` lanes the chunks use),
+// then clears the status word and the fill level on lane 0 and makes every lane wait for that.  The caller
+// holds a PipelineDrain.
+static int begin_pipeline(Context &c, const ChunkPlan &plan, uint32_t channels, size_t words_bytes, size_t ws_bytes,
+                          uint32_t lanes, PipelineViews &v)
+{
+    const size_t n_sub = (size_t)plan.start.back() * channels;
+    if (int rc = c.in.ensure(n_sub * kFrame * 2)) return rc;
+    if (int rc = c.descs.ensure(n_sub * sizeof(selab200_subframe_desc))) return rc;
+    if (int rc = c.words.ensure(words_bytes)) return rc;
+    for (uint32_t i = 0; i < lanes && i < plan.chunks(); i++)
+        if (int rc = c.lane_work[i].ensure(ws_bytes)) return rc;
+    v.status = static_cast<int32_t *>(c.small.ptr);
+    v.used = reinterpret_cast<uint64_t *>(static_cast<char *>(c.small.ptr) + 8);
+    v.pcm = static_cast<int16_t *>(c.in.ptr);
+    v.descs = static_cast<selab200_subframe_desc *>(c.descs.ptr);
+    v.words = static_cast<uint32_t *>(c.words.ptr);
+
+    CUDA_TRY(cudaMemsetAsync(c.small.ptr, 0, 16, c.s_compute[0]));
+    CUDA_TRY(cudaEventRecord(c.ev_reset, c.s_compute[0]));
+    for (int i = 1; i < kLanes; i++)
+        CUDA_TRY(cudaStreamWaitEvent(c.s_compute[i], c.ev_reset, 0));
+    return 0;
+}
+
 // The pipelined encoder over host buffers.  Two output forms: descriptors + word arena
 // (descs/words), or the byte-packed container (`container`, descs == words == nullptr) whose
-// device image lives in g.words.
-// `defer`: leave the word arena / container body on the device (g.words) instead of copying it out chunk by
+// device image lives in c.words.
+// `defer`: leave the word arena / container body on the device (c.words) instead of copying it out chunk by
 // chunk -- the multi-device driver places every device's block once the sizes of the blocks before it are known.
 // With `defer`, `container` is only a flag (any non-null value selects the byte-packed form).
-static int encode_host(const int16_t *pcm, uint32_t n_frames, uint32_t channels, selab200_subframe_desc *descs,
-                       uint32_t *words, size_t words_capacity, size_t *words_used, uint8_t *container,
-                       bool defer = false)
+static int encode_host(Context &c, const int16_t *pcm, uint32_t n_frames, uint32_t channels,
+                       selab200_subframe_desc *descs, uint32_t *words, size_t words_capacity, size_t *words_used,
+                       uint8_t *container, bool defer = false)
 {
     *words_used = 0;
     if (n_frames == 0)
         return 0;
-    PipelineDrain drain;
+    PipelineDrain drain{c};
     const ChunkPlan plan = plan_chunks(n_frames);
     const uint32_t n_chunks = plan.chunks();
-    const size_t n_sub = (size_t)n_frames * channels;
     const size_t frame_bytes = (size_t)channels * kFrame * 2;
-    const size_t ws_bytes = selab200_encode_workspace_bytes(plan.max_frames, channels);
-    if (int rc = g.in.ensure(n_sub * kFrame * 2)) return rc;
-    if (int rc = g.descs.ensure(n_sub * sizeof(selab200_subframe_desc))) return rc;
-    if (int rc = g.words.ensure(container_frame_byte(n_frames, channels, words_capacity) + 64)) return rc;
     constexpr int kEncLanes = 2;
-    for (int i = 0; i < kEncLanes && (uint32_t)i < n_chunks; i++)
-        if (int rc = g.lane_work[i].ensure(ws_bytes)) return rc;
-    int32_t *d_status = static_cast<int32_t *>(g.small.ptr);
-    uint64_t *d_used = reinterpret_cast<uint64_t *>(static_cast<char *>(g.small.ptr) + 8);
-    int16_t *d_pcm = static_cast<int16_t *>(g.in.ptr);
-    selab200_subframe_desc *d_descs = static_cast<selab200_subframe_desc *>(g.descs.ptr);
-    uint32_t *d_words = static_cast<uint32_t *>(g.words.ptr);
-
-    CUDA_TRY(cudaMemsetAsync(g.small.ptr, 0, 16, g.s_compute[0]));
-    CUDA_TRY(cudaEventRecord(g.ev_reset, g.s_compute[0]));
-    for (int i = 1; i < kLanes; i++)
-        CUDA_TRY(cudaStreamWaitEvent(g.s_compute[i], g.ev_reset, 0));
-    for (uint32_t c = 0; c < n_chunks; c++) {
-        const uint32_t f0 = plan.start[c], nf = plan.start[c + 1] - f0;
-        CUDA_TRY(cudaMemcpyAsync(d_pcm + (size_t)f0 * channels * kFrame, pcm + (size_t)f0 * channels * kFrame,
-                                 nf * frame_bytes, cudaMemcpyHostToDevice, g.s_h2d));
-        CUDA_TRY(cudaEventRecord(g.ev_h2d[c], g.s_h2d));
-        cudaStream_t cs = g.s_compute[c % kEncLanes];
-        DeviceBuffer &ws = g.lane_work[c % kEncLanes];
-        CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_h2d[c], 0));
-        if (int rc = encode_device(d_pcm + (size_t)f0 * channels * kFrame, nf, channels, d_descs + (size_t)f0 * channels,
-                                   d_words, words_capacity, d_used, d_status, ws.ptr, ws.bytes, cs, false,
-                                   c ? g.ev_scan[c - 1] : nullptr, g.ev_scan[c], &g.h_totals[c + 1],
-                                   container ? static_cast<uint8_t *>(g.words.ptr) : nullptr,
+    PipelineViews v;
+    if (int rc = begin_pipeline(c, plan, channels, container_frame_byte(n_frames, channels, words_capacity) + 64,
+                                selab200_encode_workspace_bytes(plan.max_frames, channels), kEncLanes, v))
+        return rc;
+    for (uint32_t k = 0; k < n_chunks; k++) {
+        const uint32_t f0 = plan.start[k], nf = plan.start[k + 1] - f0;
+        CUDA_TRY(cudaMemcpyAsync(v.pcm + (size_t)f0 * channels * kFrame, pcm + (size_t)f0 * channels * kFrame,
+                                 nf * frame_bytes, cudaMemcpyHostToDevice, c.s_h2d));
+        CUDA_TRY(cudaEventRecord(c.ev_h2d[k], c.s_h2d));
+        cudaStream_t cs = c.s_compute[k % kEncLanes];
+        DeviceBuffer &ws = c.lane_work[k % kEncLanes];
+        CUDA_TRY(cudaStreamWaitEvent(cs, c.ev_h2d[k], 0));
+        if (int rc = encode_device(v.pcm + (size_t)f0 * channels * kFrame, nf, channels, v.descs + (size_t)f0 * channels,
+                                   v.words, words_capacity, v.used, v.status, ws.ptr, ws.bytes, cs, false,
+                                   k ? c.ev_scan[k - 1] : nullptr, c.ev_scan[k], &c.h_totals[k + 1],
+                                   container ? static_cast<uint8_t *>(c.words.ptr) : nullptr,
                                    (unsigned long long)f0 * channels))
             return rc;
-        CUDA_TRY(cudaEventRecord(g.ev_done[c], cs));
+        CUDA_TRY(cudaEventRecord(c.ev_done[k], cs));
     }
-    g.h_totals[0] = 0;
-    for (uint32_t c = 0; c < n_chunks; c++) {
-        const uint32_t f0 = plan.start[c], nf = plan.start[c + 1] - f0;
-        CUDA_TRY(cudaEventSynchronize(g.ev_done[c]));
-        const unsigned long long lo = g.h_totals[c], hi = g.h_totals[c + 1];
+    c.h_totals[0] = 0;
+    for (uint32_t k = 0; k < n_chunks; k++) {
+        const uint32_t f0 = plan.start[k], nf = plan.start[k + 1] - f0;
+        CUDA_TRY(cudaEventSynchronize(c.ev_done[k]));
+        const unsigned long long lo = c.h_totals[k], hi = c.h_totals[k + 1];
         if (hi > words_capacity || hi < lo)
             break; // capacity exceeded: reported through the status word below
-        if (defer) {
-            if (!container)
-                CUDA_TRY(cudaMemcpyAsync(descs + (size_t)f0 * channels, d_descs + (size_t)f0 * channels,
-                                         (size_t)nf * channels * sizeof(selab200_subframe_desc), cudaMemcpyDeviceToHost,
-                                         g.s_d2h));
+        if (!container)
+            CUDA_TRY(cudaMemcpyAsync(descs + (size_t)f0 * channels, v.descs + (size_t)f0 * channels,
+                                     (size_t)nf * channels * sizeof(selab200_subframe_desc), cudaMemcpyDeviceToHost,
+                                     c.s_d2h));
+        if (defer)
             continue;
-        }
         if (container) {
             const unsigned long long b0 = container_frame_byte(f0, channels, lo);
             const unsigned long long b1 = container_frame_byte(f0 + nf, channels, hi);
-            CUDA_TRY(cudaMemcpyAsync(container + b0, static_cast<uint8_t *>(g.words.ptr) + b0, b1 - b0,
-                                     cudaMemcpyDeviceToHost, g.s_d2h));
-            continue;
+            CUDA_TRY(cudaMemcpyAsync(container + b0, static_cast<uint8_t *>(c.words.ptr) + b0, b1 - b0,
+                                     cudaMemcpyDeviceToHost, c.s_d2h));
+        } else {
+            CUDA_TRY(cudaMemcpyAsync(words + lo, v.words + lo, (hi - lo) * 4, cudaMemcpyDeviceToHost, c.s_d2h));
         }
-        CUDA_TRY(cudaMemcpyAsync(descs + (size_t)f0 * channels, d_descs + (size_t)f0 * channels,
-                                 (size_t)nf * channels * sizeof(selab200_subframe_desc), cudaMemcpyDeviceToHost,
-                                 g.s_d2h));
-        CUDA_TRY(cudaMemcpyAsync(words + lo, d_words + lo, (hi - lo) * 4, cudaMemcpyDeviceToHost, g.s_d2h));
     }
     for (int i = 0; i < kEncLanes; i++)
-        CUDA_TRY(cudaStreamSynchronize(g.s_compute[i]));
-    CUDA_TRY(cudaMemcpyAsync(g.h_small, g.small.ptr, 16, cudaMemcpyDeviceToHost, g.s_d2h));
-    CUDA_TRY(cudaStreamSynchronize(g.s_d2h));
+        CUDA_TRY(cudaStreamSynchronize(c.s_compute[i]));
+    CUDA_TRY(cudaMemcpyAsync(c.h_small, c.small.ptr, 16, cudaMemcpyDeviceToHost, c.s_d2h));
+    CUDA_TRY(cudaStreamSynchronize(c.s_d2h));
     uint64_t used;
-    memcpy(&used, g.h_small + 2, 8);
+    memcpy(&used, c.h_small + 2, 8);
     *words_used = (size_t)used; // for CAPACITY: the size the caller needs
-    if (g.h_small[0] != 0)
-        return fail(g.h_small[0], "%s", status_text(g.h_small[0]));
+    if (c.h_small[0] != 0)
+        return fail(c.h_small[0], "%s", status_text(c.h_small[0]));
     return 0;
 }
 
-static int decode_host(const selab200_subframe_desc *descs, uint32_t n_frames, uint32_t channels,
+// The chunk loop of both decode pipelines (decode_host and the container decode).  `stage(k, f0, nf, lane)`
+// brings chunk k, frames [f0, f0 + nf) of the call, onto the device: its descriptors to v.descs + f0 * channels
+// and the words they reference into the arena, with `lane` made to wait for them.  The loop decodes the chunk
+// on that lane and downloads its PCM to pcm_out, which holds the call's frames from its first.
+// Every chunk gets its own compute lane (up to kLanes): the Rice kernel is one lane per stream and
+// latency-bound (about 0.4 ms however small the chunk), so the chunks' Rice kernels must overlap
+// each other and the synthesis kernels of earlier chunks rather than queue up.
+template <typename Stage>
+static int decode_chunks(Context &c, const ChunkPlan &plan, uint32_t channels, const PipelineViews &v,
+                         const uint32_t *d_words, size_t n_words, int16_t *pcm_out, Stage stage)
+{
+    const size_t frame_bytes = (size_t)channels * kFrame * 2;
+    for (uint32_t k = 0; k < plan.chunks(); k++) {
+        const uint32_t f0 = plan.start[k], nf = plan.start[k + 1] - f0;
+        cudaStream_t cs = c.s_compute[k % kLanes];
+        DeviceBuffer &ws = c.lane_work[k % kLanes];
+        if (int rc = stage(k, f0, nf, cs))
+            return rc;
+        if (int rc = decode_device(v.descs + (size_t)f0 * channels, nf, channels, d_words, n_words,
+                                   v.pcm + (size_t)f0 * channels * kFrame, v.status, ws.ptr, ws.bytes, cs, false))
+            return rc;
+        CUDA_TRY(cudaEventRecord(c.ev_done[k], cs));
+        CUDA_TRY(cudaStreamWaitEvent(c.s_d2h, c.ev_done[k], 0));
+        CUDA_TRY(cudaMemcpyAsync(pcm_out + (size_t)f0 * channels * kFrame, v.pcm + (size_t)f0 * channels * kFrame,
+                                 nf * frame_bytes, cudaMemcpyDeviceToHost, c.s_d2h));
+    }
+    return read_status(c, c.s_d2h, v.status);
+}
+
+static int decode_host(Context &c, const selab200_subframe_desc *descs, uint32_t n_frames, uint32_t channels,
                        const uint32_t *words, size_t n_words, int16_t *pcm_out)
 {
     if (n_frames == 0)
         return 0;
-    PipelineDrain drain;
-    // Every chunk gets its own compute lane (up to kLanes): the Rice kernel is one lane per stream
-    // and latency-bound (about 0.4 ms however small the chunk), so the chunks' Rice kernels must
-    // overlap each other and the synthesis kernels of earlier chunks rather than queue up.
+    PipelineDrain drain{c};
     const ChunkPlan plan = plan_chunks(n_frames);
-    const uint32_t n_chunks = plan.chunks();
-    const size_t n_sub = (size_t)n_frames * channels;
-    const size_t frame_bytes = (size_t)channels * kFrame * 2;
-    const size_t ws_bytes = selab200_decode_workspace_bytes(plan.max_frames, channels);
-    if (int rc = g.in.ensure(n_sub * kFrame * 2)) return rc;
-    if (int rc = g.descs.ensure(n_sub * sizeof(selab200_subframe_desc))) return rc;
-    if (int rc = g.words.ensure(n_words * 4 + 16)) return rc;
-    for (int i = 0; i < kLanes && (uint32_t)i < n_chunks; i++)
-        if (int rc = g.lane_work[i].ensure(ws_bytes)) return rc;
-    int32_t *d_status = static_cast<int32_t *>(g.small.ptr);
-    int16_t *d_pcm = static_cast<int16_t *>(g.in.ptr);
-    selab200_subframe_desc *d_descs = static_cast<selab200_subframe_desc *>(g.descs.ptr);
-    uint32_t *d_words = static_cast<uint32_t *>(g.words.ptr);
-
-    CUDA_TRY(cudaMemsetAsync(g.small.ptr, 0, 16, g.s_compute[0]));
-    CUDA_TRY(cudaEventRecord(g.ev_reset, g.s_compute[0]));
-    for (int i = 1; i < kLanes; i++)
-        CUDA_TRY(cudaStreamWaitEvent(g.s_compute[i], g.ev_reset, 0));
-    for (uint32_t c = 0; c < n_chunks; c++) {
-        const uint32_t f0 = plan.start[c], nf = plan.start[c + 1] - f0;
+    PipelineViews v;
+    if (int rc = begin_pipeline(c, plan, channels, n_words * 4 + 16,
+                                selab200_decode_workspace_bytes(plan.max_frames, channels), kLanes, v))
+        return rc;
+    return decode_chunks(c, plan, channels, v, v.words, n_words, pcm_out,
+                         [&](uint32_t k, uint32_t f0, uint32_t nf, cudaStream_t cs) {
         // the words this chunk's descriptors reference (descriptors need not be in arena order)
         unsigned long long lo = ~0ull, hi = 0;
         const selab200_subframe_desc *dc = descs + (size_t)f0 * channels;
@@ -921,23 +946,14 @@ static int decode_host(const selab200_subframe_desc *descs, uint32_t n_frames, u
                 hi = b1 > hi ? b1 : hi;
             }
         }
-        CUDA_TRY(cudaMemcpyAsync(d_descs + (size_t)f0 * channels, dc, (size_t)nf * channels * sizeof(*dc),
-                                 cudaMemcpyHostToDevice, g.s_h2d));
+        CUDA_TRY(cudaMemcpyAsync(v.descs + (size_t)f0 * channels, dc, (size_t)nf * channels * sizeof(*dc),
+                                 cudaMemcpyHostToDevice, c.s_h2d));
         if (hi > lo)
-            CUDA_TRY(cudaMemcpyAsync(d_words + lo, words + lo, (hi - lo) * 4, cudaMemcpyHostToDevice, g.s_h2d));
-        CUDA_TRY(cudaEventRecord(g.ev_h2d[c], g.s_h2d));
-        cudaStream_t cs = g.s_compute[c % kLanes];
-        DeviceBuffer &ws = g.lane_work[c % kLanes];
-        CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_h2d[c], 0));
-        if (int rc = decode_device(d_descs + (size_t)f0 * channels, nf, channels, d_words, n_words,
-                                   d_pcm + (size_t)f0 * channels * kFrame, d_status, ws.ptr, ws.bytes, cs, false))
-            return rc;
-        CUDA_TRY(cudaEventRecord(g.ev_done[c], cs));
-        CUDA_TRY(cudaStreamWaitEvent(g.s_d2h, g.ev_done[c], 0));
-        CUDA_TRY(cudaMemcpyAsync(pcm_out + (size_t)f0 * channels * kFrame, d_pcm + (size_t)f0 * channels * kFrame,
-                                 nf * frame_bytes, cudaMemcpyDeviceToHost, g.s_d2h));
-    }
-    return read_status(g.s_d2h, d_status);
+            CUDA_TRY(cudaMemcpyAsync(v.words + lo, words + lo, (hi - lo) * 4, cudaMemcpyHostToDevice, c.s_h2d));
+        CUDA_TRY(cudaEventRecord(c.ev_h2d[k], c.s_h2d));
+        CUDA_TRY(cudaStreamWaitEvent(cs, c.ev_h2d[k], 0));
+        return 0;
+    });
 }
 
 // ---- every initialised device at once ----------------------------------------------------------
@@ -974,23 +990,24 @@ static bool use_all_devices(uint32_t n_frames)
     return g_n_ctx > 1 && n_frames >= 256u * (uint32_t)g_n_ctx;
 }
 
+// Runs work(context, part) for every device on a thread of its own, with that device current.
 template <typename F>
 static int run_on_devices(std::vector<DevicePart> &parts, F work)
 {
     std::vector<std::thread> threads;
     for (int d = 0; d < g_n_ctx; d++)
         threads.emplace_back([&, d] {
-            tl_ctx = &g_slots[d];
+            Context &c = g_slots[d];
             DevicePart &p = parts[d];
-            cudaError_t e = cudaSetDevice(g.device);
-            p.rc = e == cudaSuccess ? work(p) : fail(SELAB200_ERR_CUDA, "cudaSetDevice(%d) failed: %s", g.device, cudaGetErrorString(e));
+            p.rc = use_device(c);
+            if (!p.rc)
+                p.rc = work(c, p);
             if (p.rc)
                 memcpy(p.err, g_error, sizeof p.err);
         });
     for (std::thread &t : threads)
         t.join();
-    tl_ctx = &g_slots[0];
-    cudaSetDevice(g.device);
+    cudaSetDevice(g_slots[0].device);
     for (const DevicePart &p : parts)
         if (p.rc) {
             memcpy(g_error, p.err, sizeof g_error);
@@ -1004,9 +1021,9 @@ static int encode_all_devices(const int16_t *pcm, uint32_t n_frames, uint32_t ch
 {
     std::vector<DevicePart> parts = device_parts(n_frames);
     const size_t per_frame = (size_t)channels * kFrame;
-    const int rc = run_on_devices(parts, [&](DevicePart &p) {
-        return encode_host(pcm + p.f0 * per_frame, p.nf, channels, descs ? descs + (size_t)p.f0 * channels : nullptr, nullptr,
-                           selab200_encode_words_bound(p.nf, channels), &p.used, container, true);
+    const int rc = run_on_devices(parts, [&](Context &c, DevicePart &p) {
+        return encode_host(c, pcm + p.f0 * per_frame, p.nf, channels, descs ? descs + (size_t)p.f0 * channels : nullptr,
+                           nullptr, selab200_encode_words_bound(p.nf, channels), &p.used, container, true);
     });
     size_t total = 0;
     for (const DevicePart &p : parts)
@@ -1018,17 +1035,18 @@ static int encode_all_devices(const int16_t *pcm, uint32_t n_frames, uint32_t ch
         return fail(SELAB200_ERR_CAPACITY, "%s", status_text(SELAB200_ERR_CAPACITY));
     size_t base = 0;
     for (int d = 0; d < g_n_ctx; d++) { // every device's block goes out at once, each over its own link
-        tl_ctx = &g_slots[d];
+        Context &c = g_slots[d];
         const DevicePart &p = parts[d];
-        CUDA_TRY(cudaSetDevice(g.device));
+        if (int rc2 = use_device(c))
+            return rc2;
         if (container) {
             const size_t body = (size_t)container_frame_byte(p.nf, channels, p.used) - kContainerHeaderBytes;
             const size_t at = (size_t)container_frame_byte(p.f0, channels, base);
             if (body)
-                CUDA_TRY(cudaMemcpyAsync(container + at, static_cast<uint8_t *>(g.words.ptr) + kContainerHeaderBytes, body,
-                                         cudaMemcpyDeviceToHost, g.s_d2h));
+                CUDA_TRY(cudaMemcpyAsync(container + at, static_cast<uint8_t *>(c.words.ptr) + kContainerHeaderBytes, body,
+                                         cudaMemcpyDeviceToHost, c.s_d2h));
         } else if (p.used) {
-            CUDA_TRY(cudaMemcpyAsync(words + base, g.words.ptr, p.used * 4, cudaMemcpyDeviceToHost, g.s_d2h));
+            CUDA_TRY(cudaMemcpyAsync(words + base, c.words.ptr, p.used * 4, cudaMemcpyDeviceToHost, c.s_d2h));
         }
         base += p.used;
     }
@@ -1045,14 +1063,13 @@ static int encode_all_devices(const int16_t *pcm, uint32_t n_frames, uint32_t ch
     }
     int rc2 = 0;
     for (int d = 0; d < g_n_ctx; d++) {
-        tl_ctx = &g_slots[d];
-        cudaSetDevice(g.device);
-        cudaError_t e = cudaStreamSynchronize(g.s_d2h);
+        Context &c = g_slots[d];
+        cudaSetDevice(c.device);
+        cudaError_t e = cudaStreamSynchronize(c.s_d2h);
         if (e != cudaSuccess && !rc2)
-            rc2 = fail(SELAB200_ERR_CUDA, "download from device %d failed: %s", g.device, cudaGetErrorString(e));
+            rc2 = fail(SELAB200_ERR_CUDA, "download from device %d failed: %s", c.device, cudaGetErrorString(e));
     }
-    tl_ctx = &g_slots[0];
-    cudaSetDevice(g.device);
+    cudaSetDevice(g_slots[0].device);
     return rc2;
 }
 
@@ -1061,8 +1078,8 @@ static int decode_all_devices(const selab200_subframe_desc *descs, uint32_t n_fr
 {
     std::vector<DevicePart> parts = device_parts(n_frames);
     const size_t per_frame = (size_t)channels * kFrame;
-    return run_on_devices(parts, [&](DevicePart &p) {
-        return decode_host(descs + (size_t)p.f0 * channels, p.nf, channels, words, n_words, pcm_out + p.f0 * per_frame);
+    return run_on_devices(parts, [&](Context &c, DevicePart &p) {
+        return decode_host(c, descs + (size_t)p.f0 * channels, p.nf, channels, words, n_words, pcm_out + p.f0 * per_frame);
     });
 }
 
@@ -1073,15 +1090,16 @@ int selab200_encode_frames(const int16_t *pcm, uint32_t n_frames, uint32_t chann
                            size_t *words_used)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!pcm || !descs || !words || !words_used)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     if (use_all_devices(n_frames))
         return encode_all_devices(pcm, n_frames, channels, descs, words, words_capacity, words_used, nullptr);
-    return encode_host(pcm, n_frames, channels, descs, words, words_capacity, words_used, nullptr);
+    return encode_host(*c, pcm, n_frames, channels, descs, words, words_capacity, words_used, nullptr);
 }
 
 size_t selab200_container_bound(uint32_t n_frames, uint32_t channels)
@@ -1093,12 +1111,13 @@ int selab200_encode_container(const int16_t *pcm, uint32_t n_frames, uint32_t ch
                               uint16_t bits_per_sample, uint8_t *container, size_t capacity, size_t *bytes_used)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if ((!pcm && n_frames) || !container || !bytes_used)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     const unsigned long long fixed = container_frame_byte(n_frames, channels, 0);
     *bytes_used = (size_t)fixed;
     if (capacity < fixed)
@@ -1112,7 +1131,7 @@ int selab200_encode_container(const int16_t *pcm, uint32_t n_frames, uint32_t ch
     size_t words_used = 0;
     const int rc = use_all_devices(n_frames)
                        ? encode_all_devices(pcm, n_frames, channels, nullptr, nullptr, (size_t)((capacity - fixed) / 4), &words_used, container)
-                       : encode_host(pcm, n_frames, channels, nullptr, nullptr, (size_t)((capacity - fixed) / 4), &words_used, container);
+                       : encode_host(*c, pcm, n_frames, channels, nullptr, nullptr, (size_t)((capacity - fixed) / 4), &words_used, container);
     *bytes_used = (size_t)container_frame_byte(n_frames, channels, words_used);
     return rc;
 }
@@ -1121,15 +1140,16 @@ int selab200_decode_frames(const selab200_subframe_desc *descs, uint32_t n_frame
                            const uint32_t *words, size_t n_words, int16_t *pcm_out)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!descs || !pcm_out || (!words && n_words))
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     if (use_all_devices(n_frames))
         return decode_all_devices(descs, n_frames, channels, words, n_words, pcm_out);
-    return decode_host(descs, n_frames, channels, words, n_words, pcm_out);
+    return decode_host(*c, descs, n_frames, channels, words, n_words, pcm_out);
 }
 
 // ---- .sela container, decode side ----------------------------------------------------------
@@ -1241,13 +1261,13 @@ void selab200_container_close(selab200_container *h)
     if (!h)
         return;
     std::lock_guard<std::mutex> lock(g_mutex);
-    tl_ctx = &g_slots[0]; // container handles belong to the primary device
-    if (g.ready)
-        cudaSetDevice(g.device); // the caller may be on a thread that never selected the device
-    if (g.s_h2d)
-        cudaStreamSynchronize(g.s_h2d); // the upload reads the caller's bytes
-    if (g.ready && g_spare_buffers.size() < kMaxSpareBuffers)
-        g_spare_buffers.push_back(h->buf);
+    Context &c = g_slots[0]; // container handles belong to the primary device
+    if (c.ready)
+        cudaSetDevice(c.device); // the caller may be on a thread that never selected the device
+    if (c.s_h2d)
+        cudaStreamSynchronize(c.s_h2d); // the upload reads the caller's bytes
+    if (c.ready && c.spare.size() < kMaxSpareBuffers)
+        c.spare.push_back(h->buf);
     else
         h->buf.destroy();
     delete h;
@@ -1266,35 +1286,26 @@ int selab200_container_open(const uint8_t *container, size_t n_bytes, selab200_c
     int rc = 0;
     {
         std::lock_guard<std::mutex> lock(g_mutex);
-        if ((rc = require_ready()) != 0)
+        Context *c;
+        if ((rc = require_ready(c)) != 0)
             return rc;
         h = new selab200_container;
         h->bytes = container;
         h->n_bytes = n_bytes;
         // recycled buffers: the smallest spare that is large enough, else any spare (it is regrown below)
-        if (!g_spare_buffers.empty()) {
+        std::vector<ContainerBuffers> &spare = c->spare;
+        if (!spare.empty()) {
             size_t pick = 0;
-            for (size_t i = 0; i < g_spare_buffers.size(); i++)
-                if (g_spare_buffers[i].d_cap >= n_bytes + 64 &&
-                    (g_spare_buffers[pick].d_cap < n_bytes + 64 || g_spare_buffers[i].d_cap < g_spare_buffers[pick].d_cap))
+            for (size_t i = 0; i < spare.size(); i++)
+                if (spare[i].image.bytes >= n_bytes + 64 &&
+                    (spare[pick].image.bytes < n_bytes + 64 || spare[i].image.bytes < spare[pick].image.bytes))
                     pick = i;
-            h->buf = g_spare_buffers[pick];
-            g_spare_buffers.erase(g_spare_buffers.begin() + pick);
+            h->buf = spare[pick];
+            spare.erase(spare.begin() + pick);
         }
-        cudaError_t e = cudaSuccess;
-        if (h->buf.d_cap < n_bytes + 64) {
-            if (h->buf.d_bytes)
-                cudaFree(h->buf.d_bytes);
-            h->buf.d_bytes = nullptr;
-            h->buf.d_cap = 0;
-            const size_t want = n_bytes + n_bytes / 8 + 4096;
-            e = cudaMalloc(&h->buf.d_bytes, want);
-            if (e != cudaSuccess)
-                rc = fail(SELAB200_ERR_CUDA, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
-            else
-                h->buf.d_cap = want;
-        }
+        rc = h->buf.image.ensure(n_bytes + 64);
         // start the upload first: the DMA engine streams the bytes while this thread walks them
+        cudaError_t e = cudaSuccess;
         h->piece_bytes = ((n_bytes + ContainerBuffers::kPieces - 1) / ContainerBuffers::kPieces + 255) & ~(size_t)255;
         for (int i = 0; rc == 0 && (size_t)i * h->piece_bytes < n_bytes; i++) {
             const size_t lo = (size_t)i * h->piece_bytes;
@@ -1302,9 +1313,9 @@ int selab200_container_open(const uint8_t *container, size_t n_bytes, selab200_c
             if (!h->buf.ev_piece[i])
                 e = cudaEventCreateWithFlags(&h->buf.ev_piece[i], cudaEventDisableTiming);
             if (e == cudaSuccess)
-                e = cudaMemcpyAsync(static_cast<uint8_t *>(h->buf.d_bytes) + lo, container + lo, len, cudaMemcpyHostToDevice, g.s_h2d);
+                e = cudaMemcpyAsync(static_cast<uint8_t *>(h->buf.image.ptr) + lo, container + lo, len, cudaMemcpyHostToDevice, c->s_h2d);
             if (e == cudaSuccess)
-                e = cudaEventRecord(h->buf.ev_piece[i], g.s_h2d);
+                e = cudaEventRecord(h->buf.ev_piece[i], c->s_h2d);
             if (e != cudaSuccess)
                 rc = fail(SELAB200_ERR_CUDA, "container upload failed: %s", cudaGetErrorString(e));
             h->n_pieces = i + 1;
@@ -1317,28 +1328,14 @@ int selab200_container_open(const uint8_t *container, size_t n_bytes, selab200_c
         descs.reserve(n_bytes / 2048 + 16);
         rc = walk_container(container, n_bytes, &h->info, &descs);
         if (rc == 0 && !descs.empty()) {
-            if (h->buf.h_cap < descs.size()) {
-                if (h->buf.h_descs)
-                    cudaFreeHost(h->buf.h_descs);
-                h->buf.h_descs = nullptr;
-                h->buf.h_cap = 0;
-                const size_t want = descs.size() + descs.size() / 4 + 64;
-                if (cudaMallocHost(reinterpret_cast<void **>(&h->buf.h_descs), want * sizeof(selab200_subframe_desc)) != cudaSuccess)
-                    rc = fail(SELAB200_ERR_CUDA, "cudaMallocHost(%zu) failed", want * sizeof(selab200_subframe_desc));
-                else
-                    h->buf.h_cap = want;
-            }
+            const size_t bytes = descs.size() * sizeof(selab200_subframe_desc);
+            rc = h->buf.descs.ensure(bytes);
             if (rc == 0)
-                memcpy(h->buf.h_descs, descs.data(), descs.size() * sizeof(selab200_subframe_desc));
+                memcpy(h->buf.descs.ptr, descs.data(), bytes);
         }
     }
-    if (rc != 0) {
-        char keep[sizeof g_error];
-        memcpy(keep, g_error, sizeof keep);
-        selab200_container_close(h);
-        memcpy(g_error, keep, sizeof keep);
-        return rc;
-    }
+    if (rc != 0)
+        return fail_after_cleanup(rc, [h] { selab200_container_close(h); });
     *info = h->info;
     *handle = h;
     return 0;
@@ -1346,60 +1343,44 @@ int selab200_container_open(const uint8_t *container, size_t n_bytes, selab200_c
 
 } // extern "C"
 
-// Frames [F0, F0 + NF) of an open container on the device of the current context.  The primary device holds the
+// Frames [F0, F0 + NF) of an open container on the device of context `c`.  The primary device holds the
 // whole byte image (uploaded by selab200_container_open, in pieces with events); any other device uploads just
 // the bytes of its block.  The word arena keeps the descriptors' file-order offsets: it is addressed through a
 // pointer shifted back by the block's first word, so nothing is re-based.
-static int container_decode_block(selab200_container *h, uint32_t F0, uint32_t NF, int16_t *pcm_out, bool primary)
+static int container_decode_block(Context &c, selab200_container *h, uint32_t F0, uint32_t NF, int16_t *pcm_out)
 {
     if (NF == 0)
         return 0;
+    const bool primary = &c == &g_slots[0];
     const uint32_t channels = h->info.channels;
-    const selab200_subframe_desc *hd = h->buf.h_descs;
-    PipelineDrain drain;
+    const selab200_subframe_desc *hd = static_cast<const selab200_subframe_desc *>(h->buf.descs.ptr);
+    PipelineDrain drain{c};
     const ChunkPlan plan = plan_chunks(NF);
-    const uint32_t n_chunks = plan.chunks();
-    const size_t n_sub = (size_t)NF * channels;
-    const size_t frame_bytes = (size_t)channels * kFrame * 2;
-    const size_t ws_bytes = selab200_decode_workspace_bytes(plan.max_frames, channels);
-    const size_t n_words = (size_t)h->info.n_words;
     const unsigned long long w_lo = hd[(size_t)F0 * channels].refl_offset;
     const selab200_subframe_desc &tail = hd[(size_t)(F0 + NF) * channels - 1];
     const unsigned long long w_hi = tail.res_offset + tail.res_words;
-    const unsigned long long b_lo = container_frame_byte(F0, channels, w_lo);
-    const unsigned long long b_hi = container_frame_byte(F0 + NF, channels, w_hi);
-    if (int rc = g.in.ensure(n_sub * kFrame * 2)) return rc;
-    if (int rc = g.descs.ensure(n_sub * sizeof(selab200_subframe_desc))) return rc;
-    if (int rc = g.words.ensure((size_t)(w_hi - w_lo) * 4 + 96)) return rc;
-    for (int i = 0; i < kLanes && (uint32_t)i < n_chunks; i++)
-        if (int rc = g.lane_work[i].ensure(ws_bytes)) return rc;
-    int32_t *d_status = static_cast<int32_t *>(g.small.ptr);
-    int16_t *d_pcm = static_cast<int16_t *>(g.in.ptr);
-    selab200_subframe_desc *d_descs = static_cast<selab200_subframe_desc *>(g.descs.ptr);
+    PipelineViews v;
+    if (int rc = begin_pipeline(c, plan, channels, (size_t)(w_hi - w_lo) * 4 + 96,
+                                selab200_decode_workspace_bytes(plan.max_frames, channels), kLanes, v))
+        return rc;
     // 16 bytes of slack in front (the Rice decoder reads whole 16-byte vectors), the 16-byte phase of file order kept
-    uint32_t *d_arena = reinterpret_cast<uint32_t *>(static_cast<char *>(g.words.ptr) + 16 + ((w_lo * 4) & 15)) - w_lo;
-    const uint8_t *d_bytes = static_cast<const uint8_t *>(h->buf.d_bytes);
+    uint32_t *d_arena = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(v.words) + 16 + ((w_lo * 4) & 15)) - w_lo;
+    const uint8_t *d_bytes = static_cast<const uint8_t *>(h->buf.image.ptr);
     if (!primary) {
-        const unsigned long long b0 = b_lo & ~3ull; // the unpack kernel reads aligned 32-bit words of the byte image
-        const size_t end = std::min<size_t>(h->n_bytes, (size_t)b_hi + 4);
-        if (int rc = g.aux.ensure(end - (size_t)b0 + 64)) return rc;
-        CUDA_TRY(cudaMemcpyAsync(g.aux.ptr, h->bytes + b0, end - (size_t)b0, cudaMemcpyHostToDevice, g.s_h2d));
-        CUDA_TRY(cudaEventRecord(g.ev_h2d[0], g.s_h2d));
-        d_bytes = static_cast<const uint8_t *>(g.aux.ptr) - b0;
+        // the unpack kernel reads aligned 32-bit words of the byte image
+        const unsigned long long b0 = container_frame_byte(F0, channels, w_lo) & ~3ull;
+        const size_t end = std::min<size_t>(h->n_bytes, (size_t)container_frame_byte(F0 + NF, channels, w_hi) + 4);
+        if (int rc = c.aux.ensure(end - (size_t)b0 + 64)) return rc;
+        CUDA_TRY(cudaMemcpyAsync(c.aux.ptr, h->bytes + b0, end - (size_t)b0, cudaMemcpyHostToDevice, c.s_h2d));
+        CUDA_TRY(cudaEventRecord(c.ev_h2d[0], c.s_h2d));
+        d_bytes = static_cast<const uint8_t *>(c.aux.ptr) - b0;
     }
-
-    CUDA_TRY(cudaMemsetAsync(g.small.ptr, 0, 16, g.s_compute[0]));
-    CUDA_TRY(cudaEventRecord(g.ev_reset, g.s_compute[0]));
-    for (int i = 1; i < kLanes; i++)
-        CUDA_TRY(cudaStreamWaitEvent(g.s_compute[i], g.ev_reset, 0));
-    for (uint32_t c = 0; c < n_chunks; c++) {
-        const uint32_t f0 = plan.start[c], nf = plan.start[c + 1] - f0; // within the block
+    return decode_chunks(c, plan, channels, v, d_arena, (size_t)h->info.n_words, pcm_out + (size_t)F0 * channels * kFrame,
+                         [&](uint32_t, uint32_t f0, uint32_t nf, cudaStream_t cs) {
         const selab200_subframe_desc *dc = hd + (size_t)(F0 + f0) * channels;
         const size_t chunk_sub = (size_t)nf * channels;
-        cudaStream_t cs = g.s_compute[c % kLanes];
-        DeviceBuffer &ws = g.lane_work[c % kLanes];
         // descriptors go up on the chunk's own lane: s_h2d is still busy with the container bytes
-        CUDA_TRY(cudaMemcpyAsync(d_descs + (size_t)f0 * channels, dc, chunk_sub * sizeof(*dc), cudaMemcpyHostToDevice, cs));
+        CUDA_TRY(cudaMemcpyAsync(v.descs + (size_t)f0 * channels, dc, chunk_sub * sizeof(*dc), cudaMemcpyHostToDevice, cs));
         if (primary) {
             // the container bytes this chunk reads end with its last subframe (+3 bytes of slack)
             const selab200_subframe_desc &last = dc[chunk_sub - 1];
@@ -1410,22 +1391,13 @@ static int container_decode_block(selab200_container *h, uint32_t F0, uint32_t N
                 piece = h->n_pieces - 1;
             CUDA_TRY(cudaStreamWaitEvent(cs, h->buf.ev_piece[piece], 0));
         } else {
-            CUDA_TRY(cudaStreamWaitEvent(cs, g.ev_h2d[0], 0));
+            CUDA_TRY(cudaStreamWaitEvent(cs, c.ev_h2d[0], 0));
         }
-        k_container_unpack<<<(unsigned)((chunk_sub + 7) / 8), 256, 0, cs>>>(d_bytes, d_descs + (size_t)f0 * channels,
+        k_container_unpack<<<(unsigned)((chunk_sub + 7) / 8), 256, 0, cs>>>(d_bytes, v.descs + (size_t)f0 * channels,
                                                                            (uint32_t)chunk_sub, channels,
                                                                            (unsigned long long)(F0 + f0) * channels, d_arena);
-        if (int rc = launch_check("k_container_unpack"))
-            return rc;
-        if (int rc = decode_device(d_descs + (size_t)f0 * channels, nf, channels, d_arena, n_words,
-                                   d_pcm + (size_t)f0 * channels * kFrame, d_status, ws.ptr, ws.bytes, cs, false))
-            return rc;
-        CUDA_TRY(cudaEventRecord(g.ev_done[c], cs));
-        CUDA_TRY(cudaStreamWaitEvent(g.s_d2h, g.ev_done[c], 0));
-        CUDA_TRY(cudaMemcpyAsync(pcm_out + (size_t)(F0 + f0) * channels * kFrame, d_pcm + (size_t)f0 * channels * kFrame,
-                                 nf * frame_bytes, cudaMemcpyDeviceToHost, g.s_d2h));
-    }
-    return read_status(g.s_d2h, d_status);
+        return launch_check("k_container_unpack");
+    });
 }
 
 extern "C" {
@@ -1433,7 +1405,8 @@ extern "C" {
 int selab200_container_decode(selab200_container *h, int16_t *pcm_out)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!h)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
@@ -1442,30 +1415,31 @@ int selab200_container_decode(selab200_container *h, int16_t *pcm_out)
         return 0;
     if (!pcm_out)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
-    if (channels == 0 || channels > SELAB200_MAX_CHANNELS)
-        return fail(SELAB200_ERR_ARGUMENT, "channels must be in [1, %d]", SELAB200_MAX_CHANNELS);
+    if (int rc = check_channels(channels))
+        return rc;
     if (!use_all_devices(n_frames))
-        return container_decode_block(h, 0, n_frames, pcm_out, true);
+        return container_decode_block(*c, h, 0, n_frames, pcm_out);
     // one block of frames per device; the primary (which holds the whole image) takes the first
     std::vector<DevicePart> parts = device_parts(n_frames);
-    return run_on_devices(parts, [&](DevicePart &p) { return container_decode_block(h, p.f0, p.nf, pcm_out, tl_ctx == &g_slots[0]); });
+    return run_on_devices(parts, [&](Context &dc, DevicePart &p) { return container_decode_block(dc, h, p.f0, p.nf, pcm_out); });
 }
 
 int selab200_selftest(uint32_t *mismatches)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!mismatches)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
-    uint32_t *d = reinterpret_cast<uint32_t *>(static_cast<char *>(g.small.ptr) + 32);
-    CUDA_TRY(cudaMemsetAsync(d, 0, 4, g.stream));
-    k_selftest_scaling<<<(131071 + 255) / 256, 256, 0, g.stream>>>(d);
+    uint32_t *d = reinterpret_cast<uint32_t *>(static_cast<char *>(c->small.ptr) + 32);
+    CUDA_TRY(cudaMemsetAsync(d, 0, 4, c->stream));
+    k_selftest_scaling<<<(131071 + 255) / 256, 256, 0, c->stream>>>(d);
     if (int rc = launch_check("k_selftest_scaling"))
         return rc;
-    CUDA_TRY(cudaMemcpyAsync(g.h_small + 8, d, 4, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaStreamSynchronize(g.stream));
-    *mismatches = (uint32_t)g.h_small[8];
+    CUDA_TRY(cudaMemcpyAsync(c->h_small + 8, d, 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    *mismatches = (uint32_t)c->h_small[8];
     return 0;
 }
 
@@ -1474,7 +1448,8 @@ int selab200_selftest(uint32_t *mismatches)
 int selab200_lpc_residues(const int32_t *samples, uint32_t n_sub, uint8_t *order, int32_t *q, int32_t *residues)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!samples || !order || !q || !residues)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
@@ -1484,20 +1459,20 @@ int selab200_lpc_residues(const int32_t *samples, uint32_t n_sub, uint8_t *order
         if (samples[i] > 65535 || samples[i] < -65535)
             return fail(SELAB200_ERR_RANGE, "sample %zu = %d outside the 17-bit domain of 16-bit audio", i, samples[i]);
     const size_t sig = (size_t)n_sub * kFrame * 4;
-    if (int rc = g.in.ensure(sig)) return rc;
-    if (int rc = g.work.ensure(sig)) return rc;
-    if (int rc = g.aux.ensure((size_t)n_sub * kMaxOrder * 4 + n_sub + 256)) return rc;
-    int32_t *d_q = static_cast<int32_t *>(g.aux.ptr);
+    if (int rc = c->in.ensure(sig)) return rc;
+    if (int rc = c->work.ensure(sig)) return rc;
+    if (int rc = c->aux.ensure((size_t)n_sub * kMaxOrder * 4 + n_sub + 256)) return rc;
+    int32_t *d_q = static_cast<int32_t *>(c->aux.ptr);
     uint8_t *d_order = reinterpret_cast<uint8_t *>(d_q + (size_t)n_sub * kMaxOrder);
-    CUDA_TRY(cudaMemcpyAsync(g.in.ptr, samples, sig, cudaMemcpyHostToDevice, g.stream));
-    k_lpc_residues<<<n_sub, 32, 0, g.stream>>>(static_cast<const int32_t *>(g.in.ptr), n_sub, d_order, d_q,
-                                               static_cast<int32_t *>(g.work.ptr));
+    CUDA_TRY(cudaMemcpyAsync(c->in.ptr, samples, sig, cudaMemcpyHostToDevice, c->stream));
+    k_lpc_residues<<<n_sub, 32, 0, c->stream>>>(static_cast<const int32_t *>(c->in.ptr), n_sub, d_order, d_q,
+                                                static_cast<int32_t *>(c->work.ptr));
     if (int rc = launch_check("k_lpc_residues"))
         return rc;
-    CUDA_TRY(cudaMemcpyAsync(residues, g.work.ptr, sig, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(q, d_q, (size_t)n_sub * kMaxOrder * 4, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(order, d_order, n_sub, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaStreamSynchronize(g.stream));
+    CUDA_TRY(cudaMemcpyAsync(residues, c->work.ptr, sig, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(q, d_q, (size_t)n_sub * kMaxOrder * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(order, d_order, n_sub, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
     return 0;
 }
 
@@ -1505,7 +1480,8 @@ int selab200_lpc_samples(const int32_t *residues, uint32_t n_sub, const uint8_t 
                          int32_t *samples)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!residues || !order || !q || !samples)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
@@ -1515,20 +1491,20 @@ int selab200_lpc_samples(const int32_t *residues, uint32_t n_sub, const uint8_t 
         if (order[i] > kMaxOrder)
             return fail(SELAB200_ERR_BITSTREAM, "order[%u] = %u exceeds %d", i, order[i], kMaxOrder);
     const size_t sig = (size_t)n_sub * kFrame * 4;
-    if (int rc = g.in.ensure(sig)) return rc;
-    if (int rc = g.work.ensure(sig)) return rc;
-    if (int rc = g.aux.ensure((size_t)n_sub * kMaxOrder * 4 + n_sub + 256)) return rc;
-    int32_t *d_q = static_cast<int32_t *>(g.aux.ptr);
+    if (int rc = c->in.ensure(sig)) return rc;
+    if (int rc = c->work.ensure(sig)) return rc;
+    if (int rc = c->aux.ensure((size_t)n_sub * kMaxOrder * 4 + n_sub + 256)) return rc;
+    int32_t *d_q = static_cast<int32_t *>(c->aux.ptr);
     uint8_t *d_order = reinterpret_cast<uint8_t *>(d_q + (size_t)n_sub * kMaxOrder);
-    CUDA_TRY(cudaMemcpyAsync(g.in.ptr, residues, sig, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_q, q, (size_t)n_sub * kMaxOrder * 4, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_order, order, n_sub, cudaMemcpyHostToDevice, g.stream));
-    k_lpc_samples<<<n_sub, 32, 0, g.stream>>>(static_cast<const int32_t *>(g.in.ptr), n_sub, d_order, d_q,
-                                              static_cast<int32_t *>(g.work.ptr));
+    CUDA_TRY(cudaMemcpyAsync(c->in.ptr, residues, sig, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_q, q, (size_t)n_sub * kMaxOrder * 4, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_order, order, n_sub, cudaMemcpyHostToDevice, c->stream));
+    k_lpc_samples<<<n_sub, 32, 0, c->stream>>>(static_cast<const int32_t *>(c->in.ptr), n_sub, d_order, d_q,
+                                               static_cast<int32_t *>(c->work.ptr));
     if (int rc = launch_check("k_lpc_samples"))
         return rc;
-    CUDA_TRY(cudaMemcpyAsync(samples, g.work.ptr, sig, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaStreamSynchronize(g.stream));
+    CUDA_TRY(cudaMemcpyAsync(samples, c->work.ptr, sig, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
     return 0;
 }
 
@@ -1536,7 +1512,8 @@ int selab200_rice_encode(const int32_t *values, const uint32_t *counts, uint32_t
                          uint32_t *rice_param, uint32_t *n_words, uint32_t *words, uint32_t words_stride)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!values || !counts || !rice_param || !n_words || !words)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
@@ -1548,23 +1525,23 @@ int selab200_rice_encode(const int32_t *values, const uint32_t *counts, uint32_t
     if (n_streams == 0)
         return 0;
     const size_t vbytes = (size_t)n_streams * stride * 4, wbytes = (size_t)n_streams * words_stride * 4;
-    if (int rc = g.in.ensure(vbytes + 16)) return rc;
-    if (int rc = g.words.ensure(wbytes + 16)) return rc;
-    if (int rc = g.aux.ensure((size_t)n_streams * 12 + 256)) return rc;
-    uint32_t *d_counts = static_cast<uint32_t *>(g.aux.ptr);
+    if (int rc = c->in.ensure(vbytes + 16)) return rc;
+    if (int rc = c->words.ensure(wbytes + 16)) return rc;
+    if (int rc = c->aux.ensure((size_t)n_streams * 12 + 256)) return rc;
+    uint32_t *d_counts = static_cast<uint32_t *>(c->aux.ptr);
     uint32_t *d_k = d_counts + n_streams, *d_nw = d_k + n_streams;
-    int32_t *d_status = static_cast<int32_t *>(g.small.ptr);
-    CUDA_TRY(cudaMemsetAsync(d_status, 0, 4, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(g.in.ptr, values, vbytes, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_counts, counts, (size_t)n_streams * 4, cudaMemcpyHostToDevice, g.stream));
-    k_rice_encode<<<n_streams, 32, 0, g.stream>>>(static_cast<const int32_t *>(g.in.ptr), d_counts, stride, d_k,
-                                                  d_nw, static_cast<uint32_t *>(g.words.ptr), words_stride, d_status);
+    int32_t *d_status = static_cast<int32_t *>(c->small.ptr);
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, 4, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->in.ptr, values, vbytes, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_counts, counts, (size_t)n_streams * 4, cudaMemcpyHostToDevice, c->stream));
+    k_rice_encode<<<n_streams, 32, 0, c->stream>>>(static_cast<const int32_t *>(c->in.ptr), d_counts, stride, d_k,
+                                                   d_nw, static_cast<uint32_t *>(c->words.ptr), words_stride, d_status);
     if (int rc = launch_check("k_rice_encode"))
         return rc;
-    CUDA_TRY(cudaMemcpyAsync(rice_param, d_k, (size_t)n_streams * 4, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(n_words, d_nw, (size_t)n_streams * 4, cudaMemcpyDeviceToHost, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(words, g.words.ptr, wbytes, cudaMemcpyDeviceToHost, g.stream));
-    return read_status(g.stream, d_status);
+    CUDA_TRY(cudaMemcpyAsync(rice_param, d_k, (size_t)n_streams * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(n_words, d_nw, (size_t)n_streams * 4, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(words, c->words.ptr, wbytes, cudaMemcpyDeviceToHost, c->stream));
+    return read_status(*c, c->stream, d_status);
 }
 
 int selab200_rice_decode(const uint32_t *words, const uint32_t *n_words, uint32_t words_stride,
@@ -1572,32 +1549,33 @@ int selab200_rice_decode(const uint32_t *words, const uint32_t *n_words, uint32_
                          uint32_t out_stride)
 {
     std::lock_guard<std::mutex> lock(g_mutex);
-    if (int rc = require_ready())
+    Context *c;
+    if (int rc = require_ready(c))
         return rc;
     if (!words || !n_words || !rice_param || !counts || !out)
         return fail(SELAB200_ERR_ARGUMENT, "null pointer");
     if (n_streams == 0)
         return 0;
     const size_t wbytes = (size_t)n_streams * words_stride * 4, obytes = (size_t)n_streams * out_stride * 4;
-    if (int rc = g.words.ensure(wbytes + 16)) return rc;
-    if (int rc = g.work.ensure(obytes + 16)) return rc;
-    if (int rc = g.aux.ensure((size_t)n_streams * 12 + 256)) return rc;
-    uint32_t *d_nw = static_cast<uint32_t *>(g.aux.ptr);
+    if (int rc = c->words.ensure(wbytes + 16)) return rc;
+    if (int rc = c->work.ensure(obytes + 16)) return rc;
+    if (int rc = c->aux.ensure((size_t)n_streams * 12 + 256)) return rc;
+    uint32_t *d_nw = static_cast<uint32_t *>(c->aux.ptr);
     uint32_t *d_k = d_nw + n_streams, *d_counts = d_k + n_streams;
-    int32_t *d_status = static_cast<int32_t *>(g.small.ptr);
-    CUDA_TRY(cudaMemsetAsync(d_status, 0, 4, g.stream));
-    CUDA_TRY(cudaMemsetAsync(g.work.ptr, 0, obytes, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(g.words.ptr, words, wbytes, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_nw, n_words, (size_t)n_streams * 4, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_k, rice_param, (size_t)n_streams * 4, cudaMemcpyHostToDevice, g.stream));
-    CUDA_TRY(cudaMemcpyAsync(d_counts, counts, (size_t)n_streams * 4, cudaMemcpyHostToDevice, g.stream));
-    k_rice_decode_streams<<<(n_streams + 32 * kRiceWarps - 1) / (32 * kRiceWarps), 32 * kRiceWarps, 0, g.stream>>>(
-        static_cast<const uint32_t *>(g.words.ptr), d_nw, words_stride, d_k, d_counts, n_streams,
-        static_cast<int32_t *>(g.work.ptr), out_stride, d_status);
+    int32_t *d_status = static_cast<int32_t *>(c->small.ptr);
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, 4, c->stream));
+    CUDA_TRY(cudaMemsetAsync(c->work.ptr, 0, obytes, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(c->words.ptr, words, wbytes, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_nw, n_words, (size_t)n_streams * 4, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_k, rice_param, (size_t)n_streams * 4, cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_counts, counts, (size_t)n_streams * 4, cudaMemcpyHostToDevice, c->stream));
+    k_rice_decode_streams<<<(n_streams + 32 * kRiceWarps - 1) / (32 * kRiceWarps), 32 * kRiceWarps, 0, c->stream>>>(
+        static_cast<const uint32_t *>(c->words.ptr), d_nw, words_stride, d_k, d_counts, n_streams,
+        static_cast<int32_t *>(c->work.ptr), out_stride, d_status);
     if (int rc = launch_check("k_rice_decode_streams"))
         return rc;
-    CUDA_TRY(cudaMemcpyAsync(out, g.work.ptr, obytes, cudaMemcpyDeviceToHost, g.stream));
-    return read_status(g.stream, d_status);
+    CUDA_TRY(cudaMemcpyAsync(out, c->work.ptr, obytes, cudaMemcpyDeviceToHost, c->stream));
+    return read_status(*c, c->stream, d_status);
 }
 
 } // extern "C"
